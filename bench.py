@@ -2,7 +2,7 @@
 """Benchmark of the PGTG hot path (BASELINE.json: env-steps/sec, device-timed, vs CPU PGTGEnv; % HBM
 roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 A step = one fused tick (traffic, agent move, reward/termination, same-step auto-reset with
 on-device map regeneration, observation write) over every env of the rank's shard. Under torchrun
@@ -18,12 +18,17 @@ Prints ONE JSON line (rank 0):
                 in this same invocation (N = 1 only): env-steps/s, kernel ms, roofline fraction
   cpu_baseline  the CPU oracle port (C) on the host cores; cpu_baseline_python = the UNMODIFIED reference
                 PGTGEnv (oracle/_ref or /root/reference) in a forked runner, one worker per host core
+
+K sets the number of timed steps of the headline loop and of each other workload's loop. --dump-outputs DIR
+writes what the last timed step returned to its caller as DIR/<name>.npy (see dump_outputs); the inputs depend on
+the arguments alone, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
 import json
 import os
+import re
 import subprocess
 import sys
 import threading
@@ -254,6 +259,43 @@ def time_kernels_alone(env, pool, steps, flat):
     return alone
 
 
+DUMP_BUDGET = 60 * 2**20  # bytes of arrays; the rest of the 64 MiB allowed is headroom for the .npy headers
+
+
+def dump_outputs(path, step_out, flat_obs=None):
+    """Write what one `env.step` returned to its caller (observation dict, reward, terminated, truncated, info
+    dict) and, for flattened workloads, the `flat_observation` tensor, one DIR/<name>.npy per array (nested keys
+    joined with '.'). float64 arrays stay float64; everything else is written as float32, which holds its
+    small integers exactly. When all envs do not fit DUMP_BUDGET, a fixed-seed sample of envs is written, the
+    same rows of every array; env_index.npy lists them."""
+    from collections.abc import Mapping
+
+    import torch
+
+    arrays = {}
+
+    def collect(name, v):
+        if isinstance(v, Mapping):
+            for k in v:
+                collect(f"{name}.{k}", v[k])
+        elif isinstance(v, torch.Tensor):
+            arrays[re.sub(r"[^\w.-]", "_", name)] = v
+
+    for name, v in zip(("obs", "reward", "terminated", "truncated", "info"), step_out):
+        collect(name, v)
+    if flat_obs is not None:
+        collect("obs_flat", flat_obs)
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = 8 + sum(v[0].numel() * (8 if v.dtype == torch.float64 else 4) for v in arrays.values())
+    keep = min(n, DUMP_BUDGET // row_bytes)
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "env_index.npy"), idx.astype(np.float64))
+    for name, v in arrays.items():
+        rows = v.index_select(0, torch.from_numpy(idx).to(v.device)).cpu().numpy()
+        np.save(os.path.join(path, f"{name}.npy"), rows.astype(np.float64 if v.dtype == torch.float64 else np.float32))
+
+
 def measure_workload(name, dev, peak, steps=None):
     """One of the other configurations, timed in this invocation: a short device-timed loop + the kernels alone."""
     import torch
@@ -310,7 +352,10 @@ def main():
     ap.add_argument("--python-seconds", type=float, default=4.0, help="the unmodified Python reference beside the GPU path (0 = skip)")
     ap.add_argument("--no-extra", action="store_true", help="skip the other workloads")
     ap.add_argument("--final-observation", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0's envs) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     kw, n_gpu_envs, n_cpu, extras = WORKLOADS[args.workload]
     if args.envs:
         n_gpu_envs = args.envs
@@ -366,13 +411,14 @@ def main():
     ev0.record()
     for i in range(args.steps):
         kev[i][0].record()
-        env.step(pool[i % 8])
-        if flat:
-            env.flat_observation()
+        last = env.step(pool[i % 8])
+        last_flat = env.flat_observation() if flat else None
         kev[i][1].record()
     stats = env.episode_stats(all_reduce=True)  # the only collective: 8 doubles, once
     ev1.record()
     barrier()
+    if args.dump_outputs and rank == 0:  # before any further step overwrites the buffers `last` views
+        dump_outputs(args.dump_outputs, last, last_flat)
     ms = ev0.elapsed_time(ev1)
     step_ms = float(np.mean([a.elapsed_time(b) for a, b in kev]))
     ktime = env.raw.timing()
@@ -447,7 +493,7 @@ def main():
         if world == 1 and not args.no_extra and args.workload == "default-2M":
             for name in EXTRA:
                 try:
-                    workloads[name] = measure_workload(name, dev, peak)
+                    workloads[name] = measure_workload(name, dev, peak, args.steps)
                 except Exception as exc:  # keep the headline line even if an extra workload fails
                     workloads[name] = {"error": repr(exc)}
         cpu = cpu_port(kw, n_cpu, args.cpu_seconds, os.cpu_count() or 1, extras) if args.cpu_seconds > 0 else None

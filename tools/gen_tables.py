@@ -1,16 +1,18 @@
 #!/usr/bin/env python3
 """Generate the packed tile LUTs from the reference's literal tile data.
 
-Reads (never copies) /root/reference/pgtg/map_tiles_data.py (TILES :2, OBSTACLE_MASKS :1502,
-TRAFFIC_LANES :2220) and pgtg/constants.py (:18-36), checks every structural assumption the
+Reads the reference's pgtg/map_tiles_data.py (TILES :2, OBSTACLE_MASKS :1502, TRAFFIC_LANES :2220)
+from the tree named by PGTG_REFERENCE and pgtg/constants.py (:18-36), checks every structural assumption the
 kernels rely on, and emits two *differently shaped* derived tables:
 
   pgtg_b200/csrc/pgtg_tables.h   81-bit bitmaps + packed 64-bit lane descriptors (CUDA product)
   oracle/pgtg_oracle_tables.h    per-square feature words + lane lists (CPU oracle)
 
-The reference tree is absent on the GPU box, so both headers are committed; this script is the
-committed recipe that made them (`python tools/gen_tables.py`), and
-tests/test_tables.py re-derives them when /root/reference is present.
+Both headers are committed; this script is the recipe that made them (`python tools/gen_tables.py`).
+The tile data it reads is also kept as a JSON snapshot, tests/golden/tile_data.json
+(`--write-tile-data FILE` writes it from a reference tree), so that tests/test_tables.py re-derives the
+committed tables without the reference: `--tile-data FILE` reads the snapshot, `--out DIR` writes the
+three files under DIR instead of into the repository.
 
 Index conventions (shared by oracle and product, defined here once):
   tile type  e = N | E<<1 | S<<2 | W<<3          (exits list order [north,east,south,west])
@@ -22,8 +24,11 @@ Index conventions (shared by oracle and product, defined here once):
               north_and_south,east_and_west} (append order at map_generator.py:436-468)
   obstacle    1 ice, 2 broken road, 3 sand, 4 traffic_light (constants.OBSTACLE_NAMES order + 1)
 """
+import argparse
+import json
 import os
 import sys
+from types import SimpleNamespace
 
 REF = os.environ.get("PGTG_REFERENCE", "/root/reference")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -48,6 +53,45 @@ def load_reference():
     return constants, d
 
 
+def _grid(squares):
+    return [[set(c) for c in col] for col in squares]
+
+
+def load_tile_data(path):
+    """The same (constants, map_tiles_data) view as load_reference(), from a snapshot written by write_tile_data()."""
+    with open(path) as f:
+        s = json.load(f)
+    constants = SimpleNamespace(
+        TILE_WIDTH=s["TILE_WIDTH"], TILE_HEIGHT=s["TILE_HEIGHT"], OBSTACLE_NAMES=s["OBSTACLE_NAMES"],
+        OBSTACLE_MASK_NAMES=s["OBSTACLE_MASK_NAMES"], DIRECTIONS_TO_INTS=s["DIRECTIONS_TO_INTS"],
+        ACTIONS_TO_ACCELERATION={a: tuple(acc) for a, acc in s["ACTIONS_TO_ACCELERATION"]})
+    d = SimpleNamespace(
+        TILES={tuple(t["exits"]): _grid(t["squares"]) for t in s["TILES"]},
+        OBSTACLE_MASKS={name: _grid(m) for name, m in s["OBSTACLE_MASKS"].items()},
+        TRAFFIC_LANES={tuple(t["exits"]): _grid(t["squares"]) for t in s["TRAFFIC_LANES"]})
+    return constants, d
+
+
+def write_tile_data(path):
+    """Snapshot of the reference data derive() reads: feature sets as sorted lists, tiles in tile-type order."""
+    constants, d = load_reference()
+
+    def tiles(table):
+        return [dict(exits=[int(v) for v in exits], squares=[[sorted(c) for c in col] for col in t])
+                for exits, t in sorted(table.items(), key=lambda kv: type_index(kv[0]))]
+
+    s = dict(
+        TILE_WIDTH=constants.TILE_WIDTH, TILE_HEIGHT=constants.TILE_HEIGHT, OBSTACLE_NAMES=list(constants.OBSTACLE_NAMES),
+        OBSTACLE_MASK_NAMES=list(constants.OBSTACLE_MASK_NAMES), DIRECTIONS_TO_INTS=dict(constants.DIRECTIONS_TO_INTS),
+        ACTIONS_TO_ACCELERATION=[[int(a), list(acc)] for a, acc in sorted(constants.ACTIONS_TO_ACCELERATION.items())],
+        TILES=tiles(d.TILES),
+        OBSTACLE_MASKS={name: [[sorted(c) for c in col] for col in m] for name, m in d.OBSTACLE_MASKS.items()},
+        TRAFFIC_LANES=tiles(d.TRAFFIC_LANES))
+    with open(path, "w") as f:
+        json.dump(s, f, separators=(",", ":"), sort_keys=True)
+        f.write("\n")
+
+
 def type_index(exits):
     return exits[0] | exits[1] << 1 | exits[2] << 2 | exits[3] << 3
 
@@ -61,8 +105,8 @@ def bits81(pred):
     return v
 
 
-def derive():
-    constants, d = load_reference()
+def derive(tile_data=None):
+    constants, d = load_tile_data(tile_data) if tile_data else load_reference()
     assert constants.TILE_WIDTH == 9 and constants.TILE_HEIGHT == 9
     assert constants.OBSTACLE_NAMES == ["ice", "broken road", "sand", "traffic_light"]
     mask_names = list(constants.OBSTACLE_MASK_NAMES) + TL_MASKS
@@ -265,11 +309,25 @@ def emit_python(t, path):
         f.write("CARDINALS = %r\n" % (CARD,))
 
 
+OUTPUTS = ["pgtg_b200/csrc/pgtg_tables.h", "oracle/pgtg_oracle_tables.h", "pgtg_b200/_names.py"]
+
+
 def main():
-    t = derive()
-    emit_cuda(t, os.path.join(ROOT, "pgtg_b200", "csrc", "pgtg_tables.h"))
-    emit_oracle(t, os.path.join(ROOT, "oracle", "pgtg_oracle_tables.h"))
-    emit_python(t, os.path.join(ROOT, "pgtg_b200", "_names.py"))
+    ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
+    ap.add_argument("--tile-data", help="read the tile data from this JSON snapshot instead of the reference tree")
+    ap.add_argument("--write-tile-data", metavar="FILE", help="write the reference tree's tile data to FILE and exit")
+    ap.add_argument("--out", default=ROOT, help="directory the generated files are written under (default: the repository)")
+    args = ap.parse_args()
+    if args.write_tile_data:
+        write_tile_data(args.write_tile_data)
+        return
+    t = derive(args.tile_data)
+    paths = [os.path.join(args.out, p) for p in OUTPUTS]
+    for p in paths:
+        os.makedirs(os.path.dirname(p), exist_ok=True)
+    emit_cuda(t, paths[0])
+    emit_oracle(t, paths[1])
+    emit_python(t, paths[2])
     print("routes:", t["routes"])
     print("entry squares:", {k: divmod(v, 9) for k, v in t["entry_sq"].items()})
     print("exit lines:", [[divmod(i, 9) for i in range(81) if (b >> i) & 1] for b in t["exit_line"]])
