@@ -7,7 +7,6 @@
 //   int bk_h2d(void* dst, const void* src, size_t n, void* stream);   (async on stream)
 //   int bk_d2h(void* dst, const void* src, size_t n, void* stream);   (async on stream)
 //   int bk_memset(void* dst, int v, size_t n);  int bk_memset_async(void*, int, size_t, void* stream);  int bk_sync(void* stream);
-//   int bk_pick_block(const DevCfg&, int* block, size_t* smem);
 //   int bk_launch(pgtg_env*, int mode, const uint8_t* mask_dev, const int64_t* seeds_dev,
 //                 const void* actions_dev, int action_bytes, void* stream);
 //   const char* bk_error();  int bk_dl_device_type();
@@ -123,6 +122,23 @@ static void build_direction_lut(int R, std::vector<uint8_t>& lut) {
       int idx = (int)fmod((a2 + M_PI) / (M_PI / 4), 8.0);
       lut[(size_t)(dy + R) * n + (dx + R)] = (uint8_t)(o | remap[idx & 7] << 3);
     }
+}
+
+// CTA size of the tick kernel: the largest of 128 / 64 / 32 envs whose shared memory fits 200 KB (a wide sliding window
+// with many planes, or a large map, outgrows it at 128), or PGTG_BLOCK when that fits. Both backends run the
+// CTA decomposition this picks, so the emulation covers the device's smaller CTAs too.
+static int pick_block(const DevCfg& c, int* block, size_t* smem) {
+  const char* forced = getenv("PGTG_BLOCK");  // experiment knob: CTA size of the tick kernel (32 / 64 / 128)
+  int fb = forced ? atoi(forced) : 0;
+  if (fb == 32 || fb == 64 || fb == 128) {
+    size_t s = block_shared_bytes(c, fb);
+    if (s <= 200 * 1024) { *block = fb; *smem = s; return 0; }
+  }
+  for (int B : {128, 64, 32}) {
+    size_t s = block_shared_bytes(c, B);
+    if (s <= 200 * 1024) { *block = B; *smem = s; return 0; }
+  }
+  return -1;
 }
 
 // The plain configuration the LEAN tick instantiation promises (pgtg_logic.cuh, env_step): decided at
@@ -256,7 +272,7 @@ extern "C" int pgtg_create(const pgtg_config* cfg, int device, pgtg_env** out) {
   e->packed_dev = nullptr; e->stage_dev[0] = e->stage_dev[1] = nullptr; e->stage_bytes = 0; e->copy_stream = nullptr;
   e->ev_stage[0] = e->ev_stage[1] = e->ev_copied[0] = e->ev_copied[1] = nullptr; e->host_steps = 0;
   memset(&e->dp, 0, sizeof e->dp);
-  if (bk_pick_block(e->dc, &e->block, &e->smem)) { delete e; return fail(PGTG_ERR_INVALID, "observation window too large for shared memory"); }
+  if (pick_block(e->dc, &e->block, &e->smem)) { delete e; return fail(PGTG_ERR_INVALID, "observation window too large for shared memory"); }
   e->nblk = (dc.N + e->block - 1) / e->block;
   e->stats_rows = nullptr;
   e->traffic_G = e->traffic_NT = 0;

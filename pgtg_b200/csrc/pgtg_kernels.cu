@@ -52,7 +52,6 @@ static void* bk_event_create() { cudaEvent_t ev; if (ck(cudaEventCreate(&ev))) r
 static void bk_event_destroy(void* ev) { cudaEventDestroy((cudaEvent_t)ev); }
 static int bk_event_record(void* ev, void* st) { return ck(cudaEventRecord((cudaEvent_t)ev, (cudaStream_t)st)); }
 static double bk_event_elapsed(void* a, void* b) { float ms = 0; cudaEventElapsedTime(&ms, (cudaEvent_t)a, (cudaEvent_t)b); return ms; }
-static int bk_pick_block(const pgtg::DevCfg& c, int* block, size_t* smem);
 static int bk_launch(pgtg_env*, int mode, const uint8_t* mask, const int64_t* seeds, const void* actions, int action_bytes, void* stream);
 static int bk_stats_reduce(pgtg_env*, void* stream);
 static int bk_stats_reset(pgtg_env*, void* stream);
@@ -167,20 +166,6 @@ __global__ void pgtg_reduce_stats_kernel(const double* __restrict__ rows, int nr
 }  // namespace pgtg
 
 // ---- CUDA backend: launch ----------------------------------------------------------------------
-static int bk_pick_block(const pgtg::DevCfg& c, int* block, size_t* smem) {
-  const char* forced = getenv("PGTG_BLOCK");  // experiment knob: CTA size of the tick kernel (32 / 64 / 128)
-  int fb = forced ? atoi(forced) : 0;
-  if (fb == 32 || fb == 64 || fb == 128) {
-    size_t s = pgtg::block_shared_bytes(c, fb);
-    if (s <= 200 * 1024) { *block = fb; *smem = s; return 0; }
-  }
-  for (int B : {128, 64, 32}) {
-    size_t s = pgtg::block_shared_bytes(c, B);
-    if (s <= 200 * 1024) { *block = B; *smem = s; return 0; }
-  }
-  return -1;
-}
-
 // the kernel instantiations live in pgtg_inst_*.cu (one per random-number source); they return the cudaError_t
 int pgtg_launch_mode_philox(pgtg_env*, int mode, const uint8_t* mask, const int64_t* seeds, const void* actions, int action_bytes, void* stream);
 int pgtg_launch_mode_tape(pgtg_env*, int mode, const uint8_t* mask, const int64_t* seeds, const void* actions, int action_bytes, void* stream);

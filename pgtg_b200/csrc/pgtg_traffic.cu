@@ -176,7 +176,7 @@ int pgtg_traffic_geometry(const pgtg::DevCfg& c, int* G, int* NT, size_t* smem) 
   if (forced_g && (atoi(forced_g) == 32 || atoi(forced_g) == 64 || atoi(forced_g) == 128)) g = atoi(forced_g);
   const pgtg::TkLayout L = pgtg::tk_layout(c, g);
   *G = 0; *NT = 0; *smem = 0;
-  if (L.total > 220u * 1024u || c.max_cars > 0xFFFF) return 0;
+  if (!pgtg::tk_fits(c, g)) return 0;
   *G = g; *smem = L.total;
   // the per-env phases keep one warp per CTA busy: small CTAs (many per SM) while shared memory allows, one big CTA otherwise
   *NT = L.total > 72u * 1024u ? 1024 : (L.total > 28u * 1024u ? 256 : 128);

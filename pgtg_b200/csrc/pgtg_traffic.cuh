@@ -107,6 +107,9 @@ PG_HOSTDEV TkLayout tk_layout(const DevCfg& c, int G) {
   L.total = o;
   return L;
 }
+// whether the traffic tick can run a configuration with G envs per CTA; the others take the general (sequential) tick.
+// (Large maps with dense traffic, or a wide sliding window with many planes, outgrow shared memory.)
+PG_HOSTDEV bool tk_fits(const DevCfg& c, int G) { return tk_layout(c, G).total <= 220u * 1024u && c.max_cars <= 0xFFFF; }
 PG_HOSTDEV TkShared tk_carve(unsigned char* base, const TkLayout& L) {
   TkShared s;
   s.lut = (Lut*)(base + L.lut); s.spread = (uint2*)(base + L.spread); s.tiles = (uint16_t*)(base + L.tiles);

@@ -33,7 +33,6 @@ static void* bk_event_create() { return malloc(1); }
 static void bk_event_destroy(void* ev) { free(ev); }
 static int bk_event_record(void*, void*) { return 0; }
 static double bk_event_elapsed(void*, void*) { return 0.0; }
-static int bk_pick_block(const pgtg::DevCfg&, int* block, size_t* smem) { *block = 128; *smem = 0; return 0; }
 static int bk_launch(pgtg_env*, int, const uint8_t*, const int64_t*, const void*, int, void*);
 static int bk_stats_reduce(pgtg_env*, void*);
 static int bk_stats_reset(pgtg_env*, void*);
@@ -44,7 +43,8 @@ static bool bk_inline_mapgen() { return false; }
 static int bk_conn_table_max_bits() { return 13; }  // CPU tests: tables up to 8192 entries (e.g. 3x3 maps)
 static int bk_build_conn_table(pgtg_env*, uint32_t*);
 static int bk_build_path_table(pgtg_env*, uint64_t*);
-static void bk_traffic_geometry(const pgtg::DevCfg&, int* G, int* NT) { *G = 32; *NT = 96; }  // (96 emulated threads: flat loops get several rounds)
+// the device's choice between the traffic tick and the general tick; 96 emulated threads: flat loops get several rounds
+static void bk_traffic_geometry(const pgtg::DevCfg& c, int* G, int* NT) { const bool fits = pgtg::tk_fits(c, 32); *G = fits ? 32 : 0; *NT = fits ? 96 : 0; }
 
 #include "../../pgtg_b200/csrc/pgtg_api_impl.hpp"
 
