@@ -75,6 +75,8 @@ typedef enum pgtg_rng_mode {
 
 /* Draw tags on a conformance tape: stream * 8 + kind. */
 enum { PGTG_STREAM_MAP = 0, PGTG_STREAM_CAR = 1, PGTG_STREAM_ICE = 2, PGTG_STREAM_BROKEN = 3, PGTG_STREAM_SAND = 4 };
+/* Philox counter word 3 of the level draw (level sets, pgtg_levels); never a tape tag */
+enum { PGTG_STREAM_LEVEL = 5 };
 enum { PGTG_DRAW_DOUBLE = 0, PGTG_DRAW_INDEX = 1 };
 
 /* Agent heading ids used by traffic rules (environment.py:185-206). */
@@ -109,7 +111,8 @@ typedef struct pgtg_config {
   int32_t start_mode, goal_mode; /* 0: (x,y,dir) given, 1: (x,y) given, 2: "random" */
   int32_t start_x, start_y, start_dir, goal_x, goal_y, goal_dir; /* normalised (no -1), dir N0 E1 S2 W3 */
   int32_t min_start_goal_distance; /* -1 = None */
-  int32_t reserved0;
+  int32_t num_levels;  /* level set: 0 = every episode gets a fresh map; M in 1..2^24 = episodes draw one of M pre-built
+                          maps (pgtg_levels). Philox mode, procedural maps only */
   double obstacle_probability;
   double obstacle_cdf[4]; /* cumsum(p)/cumsum(p)[-1] for ice, broken road, sand, traffic_light */
 
@@ -141,14 +144,14 @@ typedef struct pgtg_config {
   int32_t separate_reward_cost;
 
   int32_t num_rules;
-  int32_t reserved1;
+  int32_t level_sampling; /* with num_levels: 0 = uniform draw per episode, 1 = env (env_id_base + i) keeps level (env_id_base + i) mod M */
   pgtg_rule rules[PGTG_MAX_RULES];
 
   /* vector-env additions (the reference gets these from wrappers: train.py:39) */
   int32_t max_episode_steps;  /* TimeLimit; 0 = none */
   int32_t write_final_obs;    /* 1: also write the terminal observation of done envs */
   int32_t max_cars;           /* capacity per env; 0 = derive from 32*W*H*density */
-  int32_t reserved2;
+  int32_t start_level;        /* with num_levels: level j is the first map of key start_level + j (0 .. 2^31 - 1) */
 } pgtg_config;
 
 /* One tile of a fixed map plan (MapPlan.tiles[y][x], map_generator.py:10-17). */
@@ -296,6 +299,17 @@ int pgtg_stats(pgtg_env* env, double* out8, int reset_after);
  * one-hots, velocity. plane_order[i] = channel index of the i-th plane in sorted-key order. The buffer is
  * allocated on first use, owned by the handle and also exported as DLPack "obs_flat". */
 int pgtg_flatten(pgtg_env* env, const int32_t* plane_order, void* stream, float** out_dev, int* out_dim);
+
+/* Level sets (num_levels > 0). Level j (0 <= j < M) is the map -- tiles, obstacles, start, goal, subgoal path -- that a
+ * handle without levels gives an env of key start_level + j at its first episode after a seeded reset; the pool is built
+ * once by pgtg_create and exported through pgtg_dlpack as "level_tiles" (uint16 [M, T], descriptor layout of
+ * pgtg_state.tiles) and "level_plan" (uint32 [M], packed start / goal / subgoal count, start-square bits clear). Episode k
+ * of env i draws its level and start square from one block philox(counter = (0, 0, k, PGTG_STREAM_LEVEL), key_i):
+ * word 0 -> level (w0 * M) >> 32 (uniform; env_index sampling uses (env_id_base + i) mod M instead), word 1 -> start
+ * square (w1 * 3) >> 32 when the start line is labelled "start" (else error flag 64). pgtg_levels writes every env's level
+ * as device int32[N] on `stream` without synchronising: of the current episode (previous = 0) or of the one before it
+ * (previous = 1: for an env that auto-reset in the last step, the episode that just ended). */
+int pgtg_levels(pgtg_env* env, int32_t* out_dev, int previous, void* stream);
 
 /* Per-kernel device timing: while enabled (max_steps > 0), pgtg_step brackets each of its kernels
  * with CUDA events on the launching stream; pgtg_timing synchronises and returns the summed

@@ -65,6 +65,7 @@ EXPORTS = {
     "pgtg_flatten": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int)]),
     "pgtg_enable_timing": (C.c_int, [C.c_void_p, C.c_int]),
     "pgtg_set_overlap": (C.c_int, [C.c_void_p, C.c_int]),
+    "pgtg_levels": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "pgtg_timing": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int)]),
 }
 

@@ -25,6 +25,8 @@ MAX_RULES = 8
 NUM_PROFILES = 5
 NUM_ROUTE_IDS = 20
 MAX_TILES = 256
+LEVELS_MAX = 1 << 24  # largest num_levels (the pool of a 16x16-tile map is then 8 GB of descriptors)
+LEVEL_SAMPLING = ("uniform", "env_index")
 
 # pgtg_channel
 CH_ZERO, CH_WALLS, CH_GOALS, CH_TRAFFIC, CH_ICE, CH_BROKEN, CH_SAND = range(7)
@@ -116,7 +118,7 @@ class PgtgConfig(C.Structure):
         ("goal_y", C.c_int32),
         ("goal_dir", C.c_int32),
         ("min_start_goal_distance", C.c_int32),
-        ("reserved0", C.c_int32),
+        ("num_levels", C.c_int32),
         ("obstacle_probability", C.c_double),
         ("obstacle_cdf", C.c_double * 4),
         ("num_channels", C.c_int32),
@@ -148,12 +150,12 @@ class PgtgConfig(C.Structure):
         ("drv_min_following", C.c_int32 * NUM_PROFILES),
         ("separate_reward_cost", C.c_int32),
         ("num_rules", C.c_int32),
-        ("reserved1", C.c_int32),
+        ("level_sampling", C.c_int32),
         ("rules", PgtgRule * MAX_RULES),
         ("max_episode_steps", C.c_int32),
         ("write_final_obs", C.c_int32),
         ("max_cars", C.c_int32),
-        ("reserved2", C.c_int32),
+        ("start_level", C.c_int32),
     ]
 
 
@@ -358,6 +360,9 @@ def make_config(
     final_observation: bool = False,
     map_plan: MapPlan | dict | None = None,
     traffic_rules: list | None = None,
+    num_levels: int = 0,
+    start_level: int = 0,
+    level_sampling: str = "uniform",
 ) -> HostConfig:
     kwargs = dict(locals())
     features = list(DEFAULT_FEATURES if features_to_include_in_observation is None else features_to_include_in_observation)
@@ -486,6 +491,19 @@ def make_config(
     for i, r in enumerate(rules):
         c.rules[i] = rule_to_pod(r)
 
+    # level sets (Procgen's num_levels / start_level): a finite pool of generated maps, built once per handle
+    if num_levels:
+        if c.rng_mode != RNG_PHILOX:
+            raise ValueError("num_levels needs rng_mode='philox'")
+        if plan is not None:
+            raise ValueError("num_levels cannot be combined with map_path / map_plan")
+        if not 1 <= int(num_levels) <= LEVELS_MAX:
+            raise ValueError(f"num_levels must be in 1..{LEVELS_MAX}")
+        if not 0 <= int(start_level) <= 2 ** 31 - 1:
+            raise ValueError("start_level must be in 0..2**31 - 1")
+        if level_sampling not in LEVEL_SAMPLING:
+            raise ValueError(f"level_sampling must be one of {LEVEL_SAMPLING}")
+        c.num_levels, c.start_level, c.level_sampling = int(num_levels), int(start_level), LEVEL_SAMPLING.index(level_sampling)
     c.max_episode_steps = 0 if not max_episode_steps else int(max_episode_steps)
     c.write_final_obs = int(bool(final_observation))
     # car capacity: lane squares per tile <= 32 (crossing), count = int(n_spawnable * density)

@@ -21,6 +21,10 @@
 //   int bk_d2d(void* dst, const void* src, size_t n, void* stream);  void* bk_stream_create();  void bk_stream_destroy(void*);
 //   int bk_info(pgtg_env*, int32_t* out_dev);  int bk_error_or(pgtg_env*, uint32_t* out_dev);   (*out_dev = OR of p.error[0..N))   (info_env for every env)
 //   void bk_traffic_geometry(const DevCfg&, int* G, int* NT);   (G = 0: the traffic tick cannot run this configuration)
+// A backend that serves level sets (pgtg_config.num_levels) also defines PGTG_BACKEND_LEVELS and
+//   int bk_serve_levels(pgtg_env*, void* stream);   (phase_serve_level over the map-request queue of launch parity dp.parity)
+//   int bk_levels(pgtg_env*, int32_t* out_dev, int previous, void* stream);   (env_level for every env)
+// without it, pgtg_create refuses num_levels > 0.
 #pragma once
 #include <math.h>
 #include <stdio.h>
@@ -35,6 +39,14 @@
 using namespace pgtg;
 
 #include "pgtg_env.hpp"
+
+#ifdef PGTG_BACKEND_LEVELS
+static const bool bk_has_levels = true;
+#else
+static const bool bk_has_levels = false;
+static int bk_serve_levels(pgtg_env*, void*) { return -1; }
+static int bk_levels(pgtg_env*, int32_t*, int, void*) { return -1; }
+#endif
 
 static thread_local std::string g_err;
 static int fail(int code, const std::string& msg) { g_err = msg; return code; }
@@ -186,6 +198,13 @@ static int fill_devcfg(const pgtg_config& c, DevCfg& d, std::string& why) {
   if (c.light_green + c.light_yellow + c.light_red <= 0 || c.light_green + c.light_yellow + c.light_red > 0x3FFF) { why = "traffic light durations out of range"; return -1; }
   if (c.rng_mode != PGTG_RNG_PHILOX && c.rng_mode != PGTG_RNG_TAPE && c.rng_mode != PGTG_RNG_NUMPY) { why = "unknown rng_mode"; return -1; }
   if (c.max_cars > 0xFFFF) { why = "max_cars too large"; return -1; }
+  if (c.num_levels) {
+    if (c.num_levels < 0 || c.num_levels > (1 << 24)) { why = "num_levels must be in 0..2^24"; return -1; }
+    if (c.rng_mode != PGTG_RNG_PHILOX) { why = "num_levels needs rng_mode = PGTG_RNG_PHILOX"; return -1; }
+    if (c.fixed_map) { why = "num_levels cannot be combined with a fixed map"; return -1; }
+    if (c.start_level < 0) { why = "start_level must be in 0..2^31 - 1"; return -1; }
+    if (c.level_sampling != 0 && c.level_sampling != 1) { why = "level_sampling must be 0 (uniform) or 1 (env index)"; return -1; }
+  }
   d.N = c.num_envs; d.W = c.map_w; d.H = c.map_h; d.T = c.map_w * c.map_h; d.WS = c.map_w * TILE; d.HS = c.map_h * TILE;
   d.C = c.num_channels; d.P = c.sliding ? 2 * c.window_k + 1 : TILE; d.sliding = c.sliding; d.window_k = c.window_k;
   d.use_nsd = c.use_next_subgoal_direction;
@@ -235,6 +254,7 @@ static int fill_devcfg(const pgtg_config& c, DevCfg& d, std::string& why) {
   d.pregen = (c.rng_mode != PGTG_RNG_TAPE && !c.fixed_map) ? 1 : 0;
   d.lean = lean_predicate(c, d);
   d.env_id_base = c.env_id_base; d.seed = c.seed;
+  d.num_levels = c.num_levels; d.level_sampling = c.level_sampling; d.start_level = c.start_level;
   if (!c.fixed_map) {
     d.n_edge_tab = 2 * (d.W * (d.H - 1) + d.H * (d.W - 1));
     d.n_border_slots = 2 * d.W + 2 * d.H - 2;
@@ -253,12 +273,67 @@ static int fill_devcfg(const pgtg_config& c, DevCfg& d, std::string& why) {
   return 0;
 }
 
+// Level sets: the pool is what the map-generation kernel builds for M pseudo-requests -- env j of a stand-in ring of M envs
+// with key start_level + j, episode 1 (the first episode after a seeded reset) -- run once on the side stream; slot 1 of that
+// ring becomes level_tiles / level_plan. The start-square bits of the plans are cleared: each episode draws its own.
+static int build_level_pool(pgtg_env* e) {
+  const size_t M = (size_t)e->cfg.num_levels, T = (size_t)e->dc.T;
+  DevPtrs& p = e->dp;
+  if (!(p.level_tiles = dev_alloc<uint16_t>(e, M * T + 8, false)) || !(p.level_plan = dev_alloc<uint32_t>(e, M, false))) return -1;
+  uint16_t* ring = (uint16_t*)bk_alloc(2 * M * T * 2 + 16);
+  uint32_t* plans = (uint32_t*)bk_alloc(2 * M * 4);
+  uint64_t* keys = (uint64_t*)bk_alloc(M * 8);
+  uint2* list = (uint2*)bk_alloc(2 * M * sizeof(uint2));
+  uint32_t* count = (uint32_t*)bk_alloc(8);
+  uint32_t* err = (uint32_t*)bk_alloc(M * 4);
+  int rc = (ring && plans && keys && list && count && err) ? 0 : -1;
+  if (!rc) {
+    std::vector<uint64_t> hk(M);
+    std::vector<uint2> hl(M);
+    for (size_t j = 0; j < M; j++) { hk[j] = (uint64_t)e->cfg.start_level + j; hl[j].x = (uint32_t)j; hl[j].y = 1u; }
+    const uint32_t hc[2] = {(uint32_t)M, 0u};
+    rc = bk_h2d(keys, hk.data(), M * 8, nullptr) || bk_h2d(list, hl.data(), M * sizeof(uint2), nullptr) || bk_h2d(count, hc, 8, nullptr) ||
+         bk_memset(err, 0, M * 4) || bk_sync(nullptr);
+  }
+  if (!rc) {
+    const DevCfg dc = e->dc;
+    const DevPtrs dp = e->dp;
+    const int grid = e->mapgen_grid;
+    e->dc.N = (int)M; e->dc.num_levels = 0;
+    e->dp.key = keys; e->dp.next_tiles = ring; e->dp.next_plan = plans; e->dp.regen_list = list; e->dp.regen_count = count;
+    e->dp.error = err; e->dp.parity = 0;
+    e->mapgen_grid = 0;
+    rc = bk_launch(e, MODE_MAPGEN, nullptr, nullptr, nullptr, 0, e->side_stream);
+    e->dc = dc; e->dp = dp; e->mapgen_grid = grid;
+    rc = rc || bk_sync(e->side_stream);
+  }
+  if (!rc) {
+    std::vector<uint32_t> hp(M);
+    rc = bk_d2d(p.level_tiles, ring + M * T, M * T * 2, nullptr) || bk_d2h(hp.data(), plans + M, M * 4, nullptr) || bk_sync(nullptr);
+    for (size_t j = 0; j < M; j++) hp[j] &= ~(3u << 29);
+    rc = rc || bk_h2d(p.level_plan, hp.data(), M * 4, nullptr) || bk_sync(nullptr);
+  }
+  for (void* a : {(void*)ring, (void*)plans, (void*)keys, (void*)list, (void*)count, (void*)err}) if (a) bk_free(a);
+  return rc;
+}
+
+// state blobs and copies carry the level set they were made with (StateHeader.reserved; 0 without levels)
+static int32_t level_fingerprint(const pgtg_config& c) {
+  if (!c.num_levels) return 0;
+  uint32_t h = 0x9E3779B9u;
+  h = (h ^ (uint32_t)c.num_levels) * 0x85EBCA6Bu;
+  h = (h ^ (uint32_t)c.start_level) * 0xC2B2AE35u;
+  h = (h ^ (uint32_t)c.level_sampling) * 0x27D4EB2Fu;
+  return (int32_t)(h | 1u);
+}
+
 extern "C" int pgtg_create(const pgtg_config* cfg, int device, pgtg_env** out) {
   if (!cfg || !out) return fail(PGTG_ERR_INVALID, "null argument");
   *out = nullptr;
   DevCfg dc;
   std::string why;
   if (fill_devcfg(*cfg, dc, why)) return fail(PGTG_ERR_INVALID, why);
+  if (cfg->num_levels && !bk_has_levels) return fail(PGTG_ERR_INVALID, "num_levels: this backend has no level sets");
   if (bk_set_device(device)) return fail(PGTG_ERR_CUDA, std::string("cannot select device: ") + bk_error());
   pgtg_env* e = new pgtg_env();
   e->cfg = *cfg; e->dc = dc; e->device = device; e->launches = 0;
@@ -408,7 +483,7 @@ extern "C" int pgtg_create(const pgtg_config* cfg, int device, pgtg_env** out) {
     int per_sm = env_ctas ? atoi(env_ctas) : 0;  // 0 = full grid (best with the connectivity table, see DESIGN.md 7)
     e->mapgen_grid = per_sm > 0 ? sms * per_sm : 0;
     e->mapgen_grid_overlap = e->mapgen_grid; e->overlap = !getenv("PGTG_NO_OVERLAP");
-    e->inline_mapgen = bk_inline_mapgen() && getenv("PGTG_INLINE_MAPGEN") != nullptr && cfg->rng_mode == PGTG_RNG_PHILOX && !getenv("PGTG_NO_LEAN");  // (and map_in_registers: below)
+    e->inline_mapgen = bk_inline_mapgen() && getenv("PGTG_INLINE_MAPGEN") != nullptr && cfg->rng_mode == PGTG_RNG_PHILOX && !getenv("PGTG_NO_LEAN") && !cfg->num_levels;  // (and map_in_registers: below)
   }
   if (e->dc.conn_bits) {
     size_t words = ((size_t)1 << e->dc.conn_bits) / 32 + 1;
@@ -438,6 +513,7 @@ extern "C" int pgtg_create(const pgtg_config* cfg, int device, pgtg_env** out) {
     p.path_table = t;
   }
   if (!pgtg::map_in_registers(e->dc)) e->inline_mapgen = false;  // (needs both tables, decided just above)
+  if (cfg->num_levels && build_level_pool(e)) { pgtg_destroy(e); return fail(PGTG_ERR_CUDA, std::string("level pool: ") + bk_error()); }
   bk_sync(nullptr);
   *out = e;
   return PGTG_OK;
@@ -559,7 +635,7 @@ static int run_pipeline(pgtg_env* e, int mode, const uint8_t* mask, const int64_
   void* ms = e->overlap ? e->side_stream : stream;  // overlap off: the generation follows the tick on the caller's stream
   if (e->overlap && (bk_event_record(e->ev_tick, stream) || bk_stream_wait(e->side_stream, e->ev_tick))) return -1;
   if (timed) bk_event_record(e->tev[e->tev_used + 2], ms);
-  if (bk_launch(e, MODE_MAPGEN, nullptr, nullptr, nullptr, 0, ms)) return -1;
+  if (e->dc.num_levels ? bk_serve_levels(e, ms) : bk_launch(e, MODE_MAPGEN, nullptr, nullptr, nullptr, 0, ms)) return -1;  // level set: the ring is filled from the pool
   e->launches++;
   if (timed) { bk_event_record(e->tev[e->tev_used + 3], ms); e->tev_used += 4; }
   if (bk_event_record(e->ev_map[par], ms)) return -1;
@@ -663,7 +739,7 @@ extern "C" int pgtg_dlpack(pgtg_env* e, const char* name, void** out) {
   const DevCfg& c = e->dc;
   const DevPtrs& p = e->dp;
   struct Spec { const char* name; void* ptr; int code, bits, ndim; int64_t shape[4]; };
-  int64_t N = c.N, C = c.C, P = c.P;
+  int64_t N = c.N, C = c.C, P = c.P, M = c.num_levels, T = c.T;
   const Spec specs[] = {
       {"obs_map", p.obs_map, 0, 8, 4, {N, C, P, P}},
       {"obs_position", p.obs_position, 0, 32, 2, {N, 2}},
@@ -681,6 +757,8 @@ extern "C" int pgtg_dlpack(pgtg_env* e, const char* name, void** out) {
       {"final_obs_next_subgoal_direction", p.f_obs_nsd, 0, 32, 1, {N}},
       {"stats", p.stats, 2, 64, 1, {8}},
       {"obs_flat", e->flat, 2, 32, 2, {N, (int64_t)e->flat_dim}},
+      {"level_tiles", p.level_tiles, 1, 16, 2, {M, T}},
+      {"level_plan", p.level_plan, 1, 32, 1, {M}},
   };
   for (const Spec& s : specs) {
     if (strcmp(s.name, name)) continue;
@@ -840,7 +918,7 @@ extern "C" int pgtg_save_state(pgtg_env* e, void* out, int64_t out_bytes) {
   if (out_bytes < pgtg_state_bytes(e)) return fail(PGTG_ERR_INVALID, "state buffer too small (see pgtg_state_bytes)");
   bk_set_device(e->device);
   if (bk_sync(nullptr)) return fail(PGTG_ERR_CUDA, std::string("device error: ") + bk_error());
-  StateHeader h = {STATE_MAGIC, (uint64_t)pgtg_state_bytes(e), e->launch_index, e->dp.parity, e->did_reset, e->cars_injected, e->dc.lean, (int32_t)e->state_allocs.size(), 0};
+  StateHeader h = {STATE_MAGIC, (uint64_t)pgtg_state_bytes(e), e->launch_index, e->dp.parity, e->did_reset, e->cars_injected, e->dc.lean, (int32_t)e->state_allocs.size(), level_fingerprint(e->cfg)};
   memcpy(out, &h, sizeof h);
   unsigned char* dst = (unsigned char*)out + sizeof h;
   for (auto& s : e->state_allocs) { bk_d2h(dst, s.ptr, s.bytes, nullptr); dst += (s.bytes + 15) & ~(size_t)15; }
@@ -855,6 +933,7 @@ extern "C" int pgtg_load_state(pgtg_env* e, const void* in, int64_t in_bytes) {
   memcpy(&h, in, sizeof h);
   if (h.magic != STATE_MAGIC || (int64_t)h.total_bytes != pgtg_state_bytes(e) || in_bytes < (int64_t)h.total_bytes || h.n_allocs != (int32_t)e->state_allocs.size())
     return fail(PGTG_ERR_INVALID, "state blob does not belong to a handle of this configuration");
+  if (h.reserved != level_fingerprint(e->cfg)) return fail(PGTG_ERR_INVALID, "state blob was saved with another level set (num_levels, start_level, level_sampling)");
   bk_set_device(e->device);
   if (bk_sync(nullptr)) return fail(PGTG_ERR_CUDA, std::string("device error: ") + bk_error());
   const unsigned char* src = (const unsigned char*)in + sizeof h;
@@ -868,6 +947,8 @@ extern "C" int pgtg_load_state(pgtg_env* e, const void* in, int64_t in_bytes) {
 extern "C" int pgtg_copy_state(pgtg_env* dst, pgtg_env* src) {
   if (!dst || !src) return fail(PGTG_ERR_INVALID, "null argument");
   if (dst->device != src->device || dst->state_allocs.size() != src->state_allocs.size()) return fail(PGTG_ERR_INVALID, "handles differ in configuration or device");
+  if (dst->cfg.num_levels != src->cfg.num_levels || dst->cfg.start_level != src->cfg.start_level || dst->cfg.level_sampling != src->cfg.level_sampling)
+    return fail(PGTG_ERR_INVALID, "handles differ in their level set (num_levels, start_level, level_sampling)");
   for (size_t i = 0; i < src->state_allocs.size(); i++)
     if (dst->state_allocs[i].bytes != src->state_allocs[i].bytes) return fail(PGTG_ERR_INVALID, "handles differ in configuration");
   bk_set_device(src->device);
@@ -1064,9 +1145,23 @@ extern "C" int64_t pgtg_launch_count(pgtg_env* e) { return e ? e->launches : 0; 
 extern "C" int pgtg_kernel_info(pgtg_env* e, char* out, int out_bytes) {
   if (!e || !out || out_bytes < 1) return fail(PGTG_ERR_INVALID, "null argument");
   const char* rng = e->cfg.rng_mode == PGTG_RNG_TAPE ? "tape" : e->cfg.rng_mode == PGTG_RNG_NUMPY ? "numpy" : "philox";
-  if (e->traffic_G > 0) snprintf(out, (size_t)out_bytes, "tick=traffic(G=%d,NT=%d) mapgen=%s rng=%s", e->traffic_G, e->traffic_NT, e->dc.pregen ? (e->dc.conn_bits && e->dc.path_tab ? "tabled" : "general") : "none", rng);
+  char levels[32];
+  snprintf(levels, sizeof levels, "levels(M=%d)", e->dc.num_levels);
+  const char* mapgen = e->dc.num_levels ? levels : e->dc.conn_bits && e->dc.path_tab ? "tabled" : "general";
+  if (e->traffic_G > 0) snprintf(out, (size_t)out_bytes, "tick=traffic(G=%d,NT=%d) mapgen=%s rng=%s", e->traffic_G, e->traffic_NT, e->dc.pregen ? mapgen : "none", rng);
   else snprintf(out, (size_t)out_bytes, "tick=%s(B=%d) mapgen=%s rng=%s", e->dc.lean && e->dc.pregen && e->cfg.rng_mode != PGTG_RNG_TAPE && !getenv("PGTG_NO_LEAN") ? (e->dc.lean == 2 ? (e->dc.write_final_obs ? "lean+slide+final" : "lean+slide") : e->dc.write_final_obs ? "lean+final" : "lean") : "general", e->block,
-                e->dc.pregen ? (e->dc.conn_bits && e->dc.path_tab ? "tabled" : "general") : "in-tick", rng);
+                e->dc.pregen ? mapgen : "in-tick", rng);
+  return PGTG_OK;
+}
+
+// Level of every env's current (previous = 0) or previous episode, device int32[N] on `stream`, no synchronisation.
+extern "C" int pgtg_levels(pgtg_env* e, int32_t* out_dev, int previous, void* stream) {
+  if (!e || !out_dev) return fail(PGTG_ERR_INVALID, "null argument");
+  if (!e->cfg.num_levels) return fail(PGTG_ERR_STATE, "config was not created with num_levels > 0");
+  if (!e->did_reset) return fail(PGTG_ERR_STATE, "levels before reset");
+  bk_set_device(e->device);
+  if (bk_levels(e, out_dev, previous != 0, stream)) return fail(PGTG_ERR_CUDA, std::string("levels launch failed: ") + bk_error());
+  e->launches++;
   return PGTG_OK;
 }
 

@@ -186,6 +186,10 @@ struct DevCfg {
   int eval_on, gamma_len;        // evaluator statistics (pgtg_set_evaluation): discounted returns with DevPtrs.gamma_pow
   int64_t env_id_base;
   uint64_t seed;
+  // level sets (pgtg_config): pool size M (0 = off), sampling (1 = level (env_id_base + env) mod M), first key of the pool.
+  // Three ints + padding = 16 bytes: the DevPtrs parameter behind this struct keeps its 16-byte alignment, so kernels that
+  // do not use levels keep their parameter loads (and the lean ticks their exact code).
+  int num_levels, level_sampling, start_level;
 };
 
 // numpy mode: one PCG64 stream (pgtg_device.cuh, 'numpy-exact generator')
@@ -254,6 +258,9 @@ struct DevPtrs {
   int32_t* step_state; uint8_t* step_flags;
   int8_t* f_obs_map; int32_t* f_obs_position; int32_t* f_obs_velocity; int32_t* f_obs_nsd;
   double* stats;
+  // level sets: the pool, built once by pgtg_create (configuration, not state)
+  uint16_t* level_tiles;  // [M][T] descriptors, no subgoal consumed
+  uint32_t* level_plan;   // [M] plan words, start-square bits clear
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -576,6 +583,31 @@ struct Rng {
     return i;
   }
 };
+
+// Level sets (specification shared with the oracle, include/pgtg_b200.h): episode k of env i takes its level and its start
+// square from ONE block philox(counter = (0, 0, k, PGTG_STREAM_LEVEL), key_i). Word 0 picks the level, (w0 * M) >> 32 (the
+// index draw of every stream); env_index sampling takes (env_id_base + i) mod M instead and leaves word 0 unused. Word 1 picks
+// the start square, (w1 * 3) >> 32, drawn only when the start line is labelled "start" (build_map's rule). The counter's
+// word 3 = 5 differs from streams 0..4 and, in its low byte, from every car-stream counter STREAM_CAR | (slot + 1) << 8, so
+// the block is no other draw's.
+PG_HD uint32_t level_draw(const DevCfg& c, uint64_t key, uint32_t episode, int env, uint32_t* start_word) {
+  uint32_t w0 = 0u, w1 = 0u, w2 = episode, w3 = (uint32_t)PGTG_STREAM_LEVEL;
+  philox4x32_10(w0, w1, w2, w3, (uint32_t)key, (uint32_t)(key >> 32));
+  *start_word = w1;
+  if (c.level_sampling) {
+    const int64_t r = (c.env_id_base + env) % (int64_t)c.num_levels;
+    return (uint32_t)(r < 0 ? r + c.num_levels : r);
+  }
+  return pg_umulhi(w0, (uint32_t)c.num_levels);
+}
+// MapView::line_labels restricted to the start line: the start tile's exit sd is labelled "start" unless the subgoal label
+// (the path leaving through that same exit) came first
+PG_HD bool start_line_labelled(unsigned start_td, unsigned plan) {
+  const int sd = plan_sd(plan), sg = td_sg(start_td);
+  const bool on_goal = plan_sy(plan) == plan_gy(plan) && plan_sx(plan) == plan_gx(plan);
+  if (!((td_exits(start_td) >> sd) & 1)) return false;
+  return !(sg && !on_goal && sg - 1 == sd);
+}
 
 // ---------------------------------------------------------------------------------------------
 // Map queries on the packed representation.

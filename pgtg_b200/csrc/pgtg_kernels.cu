@@ -58,6 +58,9 @@ static int bk_stats_reset(pgtg_env*, void* stream);
 static int bk_flatten(pgtg_env*, void* stream);
 static int bk_info(pgtg_env*, int32_t* out_dev);
 static int bk_error_or(pgtg_env*, uint32_t* out_dev);
+#define PGTG_BACKEND_LEVELS
+static int bk_serve_levels(pgtg_env*, void* stream);
+static int bk_levels(pgtg_env*, int32_t* out_dev, int previous, void* stream);
 static int bk_conn_table_max_bits() { return 24; }
 static bool bk_inline_mapgen() { return true; }
 static int bk_build_conn_table(pgtg_env*, uint32_t* table_dev);
@@ -154,6 +157,22 @@ __global__ void __launch_bounds__(256) pgtg_flatten_kernel(const __grid_constant
   }
 }
 
+// Level sets: the map-generation launch of the pipeline replaced by copies from the pool (phase_serve_level), dense over the
+// same request queue, one request per thread, grid-stride like the generator so that the persistent-grid option applies.
+__global__ void __launch_bounds__(128) pgtg_serve_levels_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ DevPtrs p, int parity) {
+  const uint32_t count = p.regen_count[parity];
+  const uint2* list = p.regen_list + (size_t)parity * 2 * c.N;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < count; i += gridDim.x * blockDim.x) {
+    const uint2 r = list[i];
+    phase_serve_level(c, p, (int)r.x, r.y);
+  }
+}
+
+// pgtg_levels: every env's level, recomputed from its key and episode counter
+__global__ void __launch_bounds__(256) pgtg_levels_kernel(const __grid_constant__ DevCfg c, const __grid_constant__ DevPtrs p, int previous, int32_t* __restrict__ out) {
+  for (int env = blockIdx.x * blockDim.x + threadIdx.x; env < c.N; env += gridDim.x * blockDim.x) out[env] = env_level(c, p, env, previous);
+}
+
 __global__ void pgtg_reduce_stats_kernel(const double* __restrict__ rows, int nrows, double* __restrict__ out) {
   // out[k] = sum over CTAs of rows[.][k]; one warp per statistic
   int k = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -227,6 +246,16 @@ static int bk_flatten(pgtg_env* e, void* stream) {
   const int blocks = want < 148 * 32 ? want : 148 * 32;
   const uint32_t pp = (uint32_t)(e->dc.P * e->dc.P), inv_pp = (uint32_t)((0x100000000ull + pp - 1) / pp);
   pgtg::pgtg_flatten_kernel<<<blocks, 32 * warps, 0, (cudaStream_t)stream>>>(e->dc, e->dp, order, e->flat, e->flat_dim, inv_pp);
+  return ck(cudaGetLastError());
+}
+static int bk_serve_levels(pgtg_env* e, void* stream) {
+  const int full = (2 * e->dc.N + 127) / 128, grid = e->mapgen_grid > 0 && e->mapgen_grid < full ? e->mapgen_grid : full;
+  pgtg::pgtg_serve_levels_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(e->dc, e->dp, e->dp.parity);
+  return ck(cudaGetLastError());
+}
+static int bk_levels(pgtg_env* e, int32_t* out_dev, int previous, void* stream) {
+  const int blocks = (e->dc.N + 255) / 256;
+  pgtg::pgtg_levels_kernel<<<blocks < 148 * 8 ? blocks : 148 * 8, 256, 0, (cudaStream_t)stream>>>(e->dc, e->dp, previous, out_dev);
   return ck(cudaGetLastError());
 }
 static int bk_stats_reset(pgtg_env* e, void* stream) {

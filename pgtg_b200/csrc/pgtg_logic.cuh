@@ -1030,8 +1030,19 @@ PG_HOSTDEV int plan_start_index(unsigned pl) { return (pl >> 29) & 3; }
 // goal / number of subgoals) and the start-square draw -- everything PGTGEnv.reset takes from
 // map_rng (environment.py:601-635). It depends only on (seed, episode), never on the actions, so
 // it can be built ahead of time by the map-generation kernel.
-template <int RNG, int TMAX, bool TABLED = false>
+// POOL = false: the generator alone (the map-generation kernel, which a level set replaces by phase_serve_level).
+template <int RNG, int TMAX, bool TABLED = false, bool POOL = true>
 PG_HD void build_map(const DevCfg& c, const DevPtrs& p, MapView& m, EnvRegs& e, Rng<RNG>& rng) {
+  if (POOL && RNG == PGTG_RNG_PHILOX && c.num_levels) {  // level set: the pool's map and the level block's start square (phase_serve_level)
+    uint32_t w1;
+    const uint32_t lv = level_draw(c, p.key[rng.env], e.episode, rng.env, &w1);
+    for (int t = 0; t < c.T; t++) m.tiles[t] = pg_ldg(&p.level_tiles[(size_t)lv * c.T + t]);
+    e.plan = pg_ldg(&p.level_plan[lv]);
+    if (start_line_labelled(m.tiles[plan_sy(e.plan) * c.W + plan_sx(e.plan)], e.plan)) e.plan |= pg_umulhi(w1, 3u) << 29;
+    else e.err |= 64;
+    m.plan = e.plan;
+    return;
+  }
   if (!TABLED && c.fixed_map) {
     for (int t = 0; t < c.T; t++) m.tiles[t] = pg_ldg(&p.fixed_tiles[t]);
     e.plan = p.fixed_plan;

@@ -67,7 +67,8 @@ def bind_to_gpu_numa_node(device_index: int, sysfs: str = "/sys/bus/pci/devices"
 
 def make_sharded(total_envs: int, device=None, bind_numa: bool = True, **kwargs):
     """A `PGTGVectorEnv` over this rank's shard of `total_envs` global envs (one process per GPU,
-    launched with torchrun)."""
+    launched with torchrun). Level sets (num_levels, start_level, level_sampling) pass through: the pool depends only on
+    the map keyword arguments and start_level, so every rank builds the same one."""
     import torch
 
     from .vector_env import PGTGVectorEnv

@@ -182,6 +182,26 @@ class RawEnv:
         _lib.check(self.lib, self.lib.pgtg_kernel_info(self._h, buf, 256))
         return buf.value.decode()
 
+    def levels(self, previous: bool = False, stream: int | None = None):
+        """Level of every env's current episode (previous=True: of the episode before it -- for an env that auto-reset in
+        the last step, the one that just ended) as a torch int32 [N] on the handle's device; no host synchronisation."""
+        import torch
+
+        if getattr(self, "_level_device", None) is None:
+            self._level_device = torch.from_dlpack(self.dlpack_capsule("level_plan")).device
+        dev = self._level_device
+        out = torch.empty(self.N, dtype=torch.int32, device=dev)
+        if stream is None:
+            stream = torch.cuda.current_stream(dev).cuda_stream if dev.type == "cuda" else 0
+        _lib.check(self.lib, self.lib.pgtg_levels(self._h, out.data_ptr(), int(bool(previous)), stream))
+        return out
+
+    def level_pool(self):
+        """-> (level_tiles uint16 [M, T], level_plan uint32 [M]) as torch views of the handle's pool."""
+        import torch
+
+        return torch.from_dlpack(self.dlpack_capsule("level_tiles")), torch.from_dlpack(self.dlpack_capsule("level_plan"))
+
     def dlpack_capsule(self, name: str):
         """-> a PyCapsule named "dltensor" for `torch.from_dlpack` / any DLPack consumer."""
         mt = C.c_void_p()

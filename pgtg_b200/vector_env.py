@@ -164,7 +164,18 @@ class PGTGVectorEnv:
             if self.hc.pod.write_final_obs:
                 info["final_observation"] = self._observation(final=True)
                 info.lazy("_final_observation", lambda: self._terminated | self._truncated)
+            if self.hc.pod.num_levels:  # the level of the episode that ended (meaningful where _final_observation is set)
+                info.lazy("final_level", lambda: self.level_ids(previous=True))
+        if self.hc.pod.num_levels:
+            info.lazy("level", self.level_ids)
         return info
+
+    def level_ids(self, previous: bool = False) -> torch.Tensor:
+        """Level sets (num_levels > 0): every env's level as int32 [N] on the device -- of the current episode, or with
+        previous=True of the episode before it, which for an env that auto-reset in the last step is the one that just ended.
+        Recomputed from the envs' keys and episode counters by one small kernel; no host synchronisation."""
+        with torch.cuda.device(self.device):
+            return self.raw.levels(previous, self._stream())
 
     def step(self, actions):
         if not self._was_reset:
