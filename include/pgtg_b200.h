@@ -251,6 +251,31 @@ int pgtg_step_host_packed(pgtg_env* env, const int32_t* actions, uint32_t* obs_p
 int pgtg_host_sync(pgtg_env* env);
 int pgtg_unpack_obs(const uint32_t* obs_packed, int8_t* obs_map, int64_t n_cells, int threads);
 
+/* Observation format (call before the first pgtg_reset; PGTG_ERR_STATE after it, PGTG_ERR_INVALID for an unknown format).
+ * PGTG_OBS_INT8, the default: every tick writes obs_map (and final_obs_map) as int8 cells. PGTG_OBS_BITS: every tick
+ * stores the planes only as bits, to the device buffer "obs_packed" (uint32 [ceil(N * C*P*P / 32)], env i at bit i * C*P*P,
+ * the layout of pgtg_step_host_packed) and, with write_final_obs, terminal observations to "final_obs_packed" (same layout;
+ * rows of envs that did not finish are not meaningful). obs_map and final_obs_map stay allocated but are written only by
+ * pgtg_expand_obs. Scalars, pgtg_step_host, pgtg_step_host_packed, pgtg_flatten, pgtg_observe, checkpoints (which then
+ * carry the bits: a blob of one format does not load into a handle of the other) and level sets work as in int8. */
+#define PGTG_OBS_INT8 0
+#define PGTG_OBS_BITS 1
+int pgtg_set_obs_format(pgtg_env* env, int format);
+/* Bits format: expand obs_packed (final != 0: final_obs_packed) into obs_map (final_obs_map) on `stream`, no synchronisation. */
+int pgtg_expand_obs(pgtg_env* env, int final, void* stream);
+/* Rows of stored bits -> int8 cells or the flattened float32 observation, on `stream`, no synchronisation (either format of
+ * the handle). bits_dev: `slots` step slots back to back, pgtg_packed_obs_bytes each (a [slots, words] tensor of obs_packed
+ * copies); row r = s * N + i is env i of slot s. index_dev: device int64 [count] rows, or NULL for rows 0 .. count - 1.
+ * PGTG_UNPACK_INT8: out_dev int8 [count, C, P, P] (32-byte aligned), cells as in obs_map. PGTG_UNPACK_FLAT: out_dev float32
+ * [count, D] in the order of pgtg_flatten (plane_order: host int32 [C], as there), position_dev / velocity_dev int32
+ * [slots, N, 2] and nsd_dev int32 [slots, N] (when next_subgoal_direction is on) gathered with the same rows. A row
+ * outside [0, slots * N) gives an all-zero output row and sets error flag 256 (pgtg_error_summary). */
+#define PGTG_UNPACK_INT8 0
+#define PGTG_UNPACK_FLAT 1
+int pgtg_unpack_bits(pgtg_env* env, const uint32_t* bits_dev, int64_t slots, const int64_t* index_dev, int64_t count, int format,
+                     void* out_dev, const int32_t* plane_order, const int32_t* position_dev, const int32_t* velocity_dev,
+                     const int32_t* nsd_dev, void* stream);
+
 /* Recompute the observation buffers from the current state without ticking (the second half of
  * set_to_state, environment.py:1342). */
 int pgtg_observe(pgtg_env* env, void* stream);
@@ -320,7 +345,8 @@ int pgtg_enable_timing(pgtg_env* env, int max_steps);
 int pgtg_set_overlap(pgtg_env* env, int on);
 int pgtg_timing(pgtg_env* env, double* tick_ms, double* mapgen_ms, int* steps);
 /* OR of every env's sticky error flags (bit 7 = 128: an action outside 0..8 was replaced by the no-op 4, where the
- * reference raises KeyError; the other bits are listed in pgtg_api_impl.hpp). Synchronises. */
+ * reference raises KeyError; the other bits are listed in pgtg_api_impl.hpp) and of the handle's (bit 8 = 256: a
+ * pgtg_unpack_bits index out of range). Synchronises. */
 int pgtg_error_summary(pgtg_env* env, uint32_t* out_flags);
 /* Number of kernels this handle has launched so far (bench.py's gpu_launches). */
 int64_t pgtg_launch_count(pgtg_env* env);

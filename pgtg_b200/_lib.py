@@ -13,6 +13,9 @@ from .config import PgtgConfig, PgtgRule, PgtgTile
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpgtg_b200.so")
 
+OBS_FORMATS = {"int8": 0, "bits": 1}  # PGTG_OBS_INT8 / PGTG_OBS_BITS
+UNPACK_FORMATS = {"int8": 0, "flat": 1}  # PGTG_UNPACK_INT8 / PGTG_UNPACK_FLAT
+
 STATE_FIELDS = ("agent", "flat_tire", "light_counter", "elapsed", "num_cars", "cars", "tiles", "plan", "used",
                 "draw_cursor", "error")
 
@@ -66,6 +69,9 @@ EXPORTS = {
     "pgtg_enable_timing": (C.c_int, [C.c_void_p, C.c_int]),
     "pgtg_set_overlap": (C.c_int, [C.c_void_p, C.c_int]),
     "pgtg_levels": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "pgtg_set_obs_format": (C.c_int, [C.c_void_p, C.c_int]),
+    "pgtg_expand_obs": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "pgtg_unpack_bits": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int] + [C.c_void_p] * 6),
     "pgtg_timing": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int)]),
 }
 

@@ -25,6 +25,8 @@ MAX_RULES = 8
 NUM_PROFILES = 5
 NUM_ROUTE_IDS = 20
 MAX_TILES = 256
+# observation planes as stored by the ticks: int8 cells [N, C, P, P], or bits (env i at bit i * C*P*P; pgtg_set_obs_format)
+OBSERVATION_FORMATS = ("int8", "bits")
 LEVELS_MAX = 1 << 24  # largest num_levels (the pool of a 16x16-tile map is then 8 GB of descriptors)
 LEVEL_SAMPLING = ("uniform", "env_index")
 
@@ -217,6 +219,7 @@ class HostConfig:
     window: int
     map_plan: MapPlan | None = None
     rules: list = field(default_factory=list)
+    observation_format: str = "int8"  # how the ticks store the observation planes: int8 cells or bits (pgtg_set_obs_format)
 
 
 def _validate_generate_map_args(width, height, start_position, goal_position, min_dist):
@@ -363,6 +366,7 @@ def make_config(
     num_levels: int = 0,
     start_level: int = 0,
     level_sampling: str = "uniform",
+    observation_format: str = "int8",
 ) -> HostConfig:
     kwargs = dict(locals())
     features = list(DEFAULT_FEATURES if features_to_include_in_observation is None else features_to_include_in_observation)
@@ -504,6 +508,8 @@ def make_config(
         if level_sampling not in LEVEL_SAMPLING:
             raise ValueError(f"level_sampling must be one of {LEVEL_SAMPLING}")
         c.num_levels, c.start_level, c.level_sampling = int(num_levels), int(start_level), LEVEL_SAMPLING.index(level_sampling)
+    if observation_format not in OBSERVATION_FORMATS:
+        raise ValueError(f"observation_format must be one of {OBSERVATION_FORMATS}")
     c.max_episode_steps = 0 if not max_episode_steps else int(max_episode_steps)
     c.write_final_obs = int(bool(final_observation))
     # car capacity: lane squares per tile <= 32 (crossing), count = int(n_spawnable * density)
@@ -511,7 +517,8 @@ def make_config(
         c.max_cars = max(1, int(32 * W * H * min(float(traffic_density), 1.0)))
     else:
         c.max_cars = 1
-    return HostConfig(pod=c, kwargs=kwargs, observation_keys=[k for k, _ in layout], window=window, map_plan=plan, rules=rules)
+    return HostConfig(pod=c, kwargs=kwargs, observation_keys=[k for k, _ in layout], window=window, map_plan=plan, rules=rules,
+                      observation_format=observation_format)
 
 
 def direction_lut(radius: int) -> np.ndarray:

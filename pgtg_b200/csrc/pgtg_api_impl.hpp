@@ -25,6 +25,10 @@
 //   int bk_serve_levels(pgtg_env*, void* stream);   (phase_serve_level over the map-request queue of launch parity dp.parity)
 //   int bk_levels(pgtg_env*, int32_t* out_dev, int previous, void* stream);   (env_level for every env)
 // without it, pgtg_create refuses num_levels > 0.
+// A backend with the bits observation format (pgtg_set_obs_format) also defines PGTG_BACKEND_OBS_BITS and
+//   int bk_unpack_bits(pgtg_env*, const UnpackArgs&, int format, void* out_dev, const int* plane_order, void* stream);
+//       (unpack_chunk / unpack_flat_cell / unpack_flat_tail over the rows of a; PGTG_UNPACK_INT8 or PGTG_UNPACK_FLAT)
+// without it, pgtg_set_obs_format refuses PGTG_OBS_BITS and pgtg_unpack_bits fails.
 #pragma once
 #include <math.h>
 #include <stdio.h>
@@ -46,6 +50,12 @@ static const bool bk_has_levels = true;
 static const bool bk_has_levels = false;
 static int bk_serve_levels(pgtg_env*, void*) { return -1; }
 static int bk_levels(pgtg_env*, int32_t*, int, void*) { return -1; }
+#endif
+#ifdef PGTG_BACKEND_OBS_BITS
+static const bool bk_has_obs_bits = true;
+#else
+static const bool bk_has_obs_bits = false;
+static int bk_unpack_bits(pgtg_env*, const UnpackArgs&, int, void*, const int*, void*) { return -1; }
 #endif
 
 static thread_local std::string g_err;
@@ -346,6 +356,7 @@ extern "C" int pgtg_create(const pgtg_config* cfg, int device, pgtg_env** out) {
   e->info_dev = nullptr;
   e->packed_dev = nullptr; e->stage_dev[0] = e->stage_dev[1] = nullptr; e->stage_bytes = 0; e->copy_stream = nullptr;
   e->ev_stage[0] = e->ev_stage[1] = e->ev_copied[0] = e->ev_copied[1] = nullptr; e->host_steps = 0;
+  e->obs_format = PGTG_OBS_INT8; e->obs_map_buf = e->f_obs_map_buf = nullptr; e->obs_packed_buf = e->f_obs_packed_buf = nullptr;
   memset(&e->dp, 0, sizeof e->dp);
   if (pick_block(e->dc, &e->block, &e->smem)) { delete e; return fail(PGTG_ERR_INVALID, "observation window too large for shared memory"); }
   e->nblk = (dc.N + e->block - 1) / e->block;
@@ -381,6 +392,7 @@ extern "C" int pgtg_create(const pgtg_config* cfg, int device, pgtg_env** out) {
   ok = ok && ((e->mask_dev = dev_alloc<uint8_t>(e, N)) != nullptr);
   ok = ok && ((e->seeds_dev = dev_alloc<int64_t>(e, N)) != nullptr);
   ok = ok && ((e->actions_dev = dev_alloc<int32_t>(e, N)) != nullptr);
+  ok = ok && ((e->unpack_err = dev_alloc<uint32_t>(e, 1)) != nullptr);
 #undef A
   if (!ok) { pgtg_destroy(e); return fail(PGTG_ERR_CUDA, std::string("device allocation failed: ") + bk_error()); }
   // next_subgoal_direction is -1 when the feature is off (environment.py:1358)
@@ -695,6 +707,12 @@ extern "C" int pgtg_step(pgtg_env* e, const void* actions_dev, int action_bytes,
   return PGTG_OK;
 }
 
+// the int8 planes (final: terminal observations) whatever the format: in bits mode written only by pgtg_expand_obs
+static int8_t* obs_map_of(const pgtg_env* e, bool final) {
+  if (e->obs_format == PGTG_OBS_BITS) return final ? e->f_obs_map_buf : e->obs_map_buf;
+  return final ? e->dp.f_obs_map : e->dp.obs_map;
+}
+
 extern "C" int pgtg_step_host(pgtg_env* e, const int32_t* actions, int8_t* obs_map, int32_t* obs_position,
                               int32_t* obs_velocity, double* reward, uint8_t* terminated, uint8_t* truncated, void* stream) {
   if (!e || !actions) return fail(PGTG_ERR_INVALID, "null argument");
@@ -703,7 +721,8 @@ extern "C" int pgtg_step_host(pgtg_env* e, const int32_t* actions, int8_t* obs_m
   bk_h2d(e->actions_dev, actions, N * 4, stream);
   int rc = pgtg_step(e, e->actions_dev, 4, stream);
   if (rc) return rc;
-  if (obs_map) bk_d2h(obs_map, e->dp.obs_map, N * e->dc.obs_bits, stream);
+  if (obs_map && e->obs_format == PGTG_OBS_BITS && (rc = pgtg_expand_obs(e, 0, stream))) return rc;
+  if (obs_map) bk_d2h(obs_map, obs_map_of(e, false), N * e->dc.obs_bits, stream);
   if (obs_position) bk_d2h(obs_position, e->dp.obs_position, N * 8, stream);
   if (obs_velocity) bk_d2h(obs_velocity, e->dp.obs_velocity, N * 8, stream);
   if (reward) bk_d2h(reward, e->dp.reward, N * 8, stream);
@@ -718,10 +737,10 @@ extern "C" int pgtg_get_buffers(pgtg_env* e, pgtg_buffers* out) {
   memset(out, 0, sizeof *out);
   const DevPtrs& p = e->dp;
   out->num_envs = e->dc.N; out->num_channels = e->dc.C; out->window = e->dc.P; out->max_cars = e->dc.max_cars;
-  out->obs_map = p.obs_map; out->obs_position = p.obs_position; out->obs_velocity = p.obs_velocity;
+  out->obs_map = obs_map_of(e, false); out->obs_position = p.obs_position; out->obs_velocity = p.obs_velocity;
   out->obs_next_subgoal_direction = p.obs_nsd; out->reward = p.reward; out->cost = p.cost;
   out->terminated = p.terminated; out->truncated = p.truncated; out->step_state = p.step_state; out->step_flags = p.step_flags;
-  out->final_obs_map = p.f_obs_map; out->final_obs_position = p.f_obs_position; out->final_obs_velocity = p.f_obs_velocity;
+  out->final_obs_map = obs_map_of(e, true); out->final_obs_position = p.f_obs_position; out->final_obs_velocity = p.f_obs_velocity;
   out->final_obs_next_subgoal_direction = p.f_obs_nsd; out->stats = p.stats;
   return PGTG_OK;
 }
@@ -739,9 +758,9 @@ extern "C" int pgtg_dlpack(pgtg_env* e, const char* name, void** out) {
   const DevCfg& c = e->dc;
   const DevPtrs& p = e->dp;
   struct Spec { const char* name; void* ptr; int code, bits, ndim; int64_t shape[4]; };
-  int64_t N = c.N, C = c.C, P = c.P, M = c.num_levels, T = c.T;
+  int64_t N = c.N, C = c.C, P = c.P, M = c.num_levels, T = c.T, W = pgtg_packed_obs_bytes(e) / 4;
   const Spec specs[] = {
-      {"obs_map", p.obs_map, 0, 8, 4, {N, C, P, P}},
+      {"obs_map", obs_map_of(e, false), 0, 8, 4, {N, C, P, P}},
       {"obs_position", p.obs_position, 0, 32, 2, {N, 2}},
       {"obs_velocity", p.obs_velocity, 0, 32, 2, {N, 2}},
       {"obs_next_subgoal_direction", p.obs_nsd, 0, 32, 1, {N}},
@@ -751,7 +770,7 @@ extern "C" int pgtg_dlpack(pgtg_env* e, const char* name, void** out) {
       {"truncated", p.truncated, 1, 8, 1, {N}},
       {"step_state", p.step_state, 0, 32, 2, {N, 4}},
       {"step_flags", p.step_flags, 1, 8, 1, {N}},
-      {"final_obs_map", p.f_obs_map, 0, 8, 4, {N, C, P, P}},
+      {"final_obs_map", obs_map_of(e, true), 0, 8, 4, {N, C, P, P}},
       {"final_obs_position", p.f_obs_position, 0, 32, 2, {N, 2}},
       {"final_obs_velocity", p.f_obs_velocity, 0, 32, 2, {N, 2}},
       {"final_obs_next_subgoal_direction", p.f_obs_nsd, 0, 32, 1, {N}},
@@ -759,6 +778,8 @@ extern "C" int pgtg_dlpack(pgtg_env* e, const char* name, void** out) {
       {"obs_flat", e->flat, 2, 32, 2, {N, (int64_t)e->flat_dim}},
       {"level_tiles", p.level_tiles, 1, 16, 2, {M, T}},
       {"level_plan", p.level_plan, 1, 32, 1, {M}},
+      {"obs_packed", p.obs_packed, 1, 32, 1, {W}},
+      {"final_obs_packed", p.f_obs_packed, 1, 32, 1, {W}},
   };
   for (const Spec& s : specs) {
     if (strcmp(s.name, name)) continue;
@@ -1008,8 +1029,8 @@ extern "C" int pgtg_step_host_packed(pgtg_env* e, const int32_t* actions, uint32
   bk_set_device(e->device);
   const size_t N = (size_t)e->dc.N;
   const HostLayout L = host_layout(e);
-  if (!e->packed_dev) {
-    e->packed_dev = dev_alloc<uint32_t>(e, (size_t)pgtg_packed_obs_bytes(e) / 4 + 8);
+  if (!e->stage_dev[0]) {  // (in bits mode the ticks store obs_packed anyway: no buffer of its own)
+    e->packed_dev = e->dp.obs_packed ? e->dp.obs_packed : dev_alloc<uint32_t>(e, (size_t)pgtg_packed_obs_bytes(e) / 4 + 8);
     e->stage_dev[0] = dev_alloc<unsigned char>(e, L.total); e->stage_dev[1] = dev_alloc<unsigned char>(e, L.total);
     e->copy_stream = bk_stream_create();
     for (int i = 0; i < 2; i++) { e->ev_stage[i] = bk_event_create(); e->ev_copied[i] = bk_event_create(); }
@@ -1118,7 +1139,11 @@ extern "C" int pgtg_flatten(pgtg_env* e, const int32_t* plane_order, void* strea
     if (plane_order[i] < 0 || plane_order[i] >= c.C) return fail(PGTG_ERR_INVALID, "bad plane order");
     e->flat_order[i] = plane_order[i];
   }
-  if (bk_flatten(e, stream)) return fail(PGTG_ERR_CUDA, std::string("flatten launch failed: ") + bk_error());
+  if (e->obs_format == PGTG_OBS_BITS) {  // straight from the bits: the unpack kernel over the current step's rows
+    const int rc = pgtg_unpack_bits(e, e->dp.obs_packed, 1, nullptr, c.N, PGTG_UNPACK_FLAT, e->flat, plane_order, e->dp.obs_position,
+                                    e->dp.obs_velocity, e->dp.obs_nsd, stream);
+    if (rc) return rc;
+  } else if (bk_flatten(e, stream)) return fail(PGTG_ERR_CUDA, std::string("flatten launch failed: ") + bk_error());
   e->launches++;
   if (out_dev) *out_dev = e->flat;
   if (out_dim) *out_dim = dim;
@@ -1126,7 +1151,8 @@ extern "C" int pgtg_flatten(pgtg_env* e, const int32_t* plane_order, void* strea
 }
 
 // OR of every env's sticky error flags (1 tape overrun, 2 tape tag mismatch, 4 tape index out of range, 8 goal unreachable,
-// 16 no route at a spawn square, 32 more cars than max_cars, 64 no start square, 128 action outside 0..8). Synchronises.
+// 16 no route at a spawn square, 32 more cars than max_cars, 64 no start square, 128 action outside 0..8) and of the handle's
+// (256 a pgtg_unpack_bits index out of range). Synchronises.
 extern "C" int pgtg_error_summary(pgtg_env* e, uint32_t* out_flags) {
   if (!e || !out_flags) return fail(PGTG_ERR_INVALID, "null argument");
   bk_set_device(e->device);
@@ -1134,9 +1160,78 @@ extern "C" int pgtg_error_summary(pgtg_env* e, uint32_t* out_flags) {
   if (!e->info_dev && !(e->info_dev = dev_alloc<int32_t>(e, 7 * (size_t)e->dc.N))) return fail(PGTG_ERR_CUDA, std::string("device allocation failed: ") + bk_error());
   if (bk_error_or(e, (uint32_t*)e->info_dev)) return fail(PGTG_ERR_CUDA, std::string("launch failed: ") + bk_error());
   e->launches++;
+  uint32_t handle_flags = 0;
   bk_d2h(out_flags, e->info_dev, 4, nullptr);
+  bk_d2h(&handle_flags, e->unpack_err, 4, nullptr);
   if (bk_sync(nullptr)) return fail(PGTG_ERR_CUDA, std::string("device error: ") + bk_error());
+  *out_flags |= handle_flags;
   return PGTG_OK;
+}
+
+// ---- bits observation format ----------------------------------------------------------------------------------------------
+extern "C" int pgtg_set_obs_format(pgtg_env* e, int format) {
+  if (!e) return fail(PGTG_ERR_INVALID, "null handle");
+  if (format != PGTG_OBS_INT8 && format != PGTG_OBS_BITS) return fail(PGTG_ERR_INVALID, "unknown observation format (PGTG_OBS_INT8 or PGTG_OBS_BITS)");
+  if (e->did_reset) return fail(PGTG_ERR_STATE, "the observation format can only be set before the first pgtg_reset");
+  if (format == PGTG_OBS_BITS && !bk_has_obs_bits) return fail(PGTG_ERR_INVALID, "this backend has no bits observation format");
+  if (format == e->obs_format) return PGTG_OK;
+  bk_set_device(e->device);
+  DevPtrs& p = e->dp;
+  const size_t bytes = (size_t)pgtg_packed_obs_bytes(e);
+  if (format == PGTG_OBS_BITS) {
+    if (!e->obs_packed_buf && !(e->obs_packed_buf = dev_alloc<uint32_t>(e, bytes / 4 + 8))) return fail(PGTG_ERR_CUDA, std::string("device allocation failed: ") + bk_error());
+    if (e->dc.write_final_obs && !e->f_obs_packed_buf && !(e->f_obs_packed_buf = dev_alloc<uint32_t>(e, bytes / 4 + 8)))
+      return fail(PGTG_ERR_CUDA, std::string("device allocation failed: ") + bk_error());
+    // checkpoints carry the bits (the int8 buffers stay state allocations too: a blob of the other format has another size)
+    e->state_allocs.push_back({e->obs_packed_buf, bytes});
+    if (e->f_obs_packed_buf) e->state_allocs.push_back({e->f_obs_packed_buf, bytes});
+    e->obs_map_buf = p.obs_map; e->f_obs_map_buf = p.f_obs_map;
+    p.obs_map = nullptr; p.f_obs_map = nullptr;
+    p.obs_packed = e->obs_packed_buf; p.f_obs_packed = e->f_obs_packed_buf;
+  } else {
+    for (void* b : {(void*)e->obs_packed_buf, (void*)e->f_obs_packed_buf})
+      for (size_t i = 0; i < e->state_allocs.size(); i++)
+        if (b && e->state_allocs[i].ptr == b) { e->state_allocs.erase(e->state_allocs.begin() + i); break; }
+    p.obs_map = e->obs_map_buf; p.f_obs_map = e->f_obs_map_buf;
+    p.obs_packed = nullptr; p.f_obs_packed = nullptr;  // (no host-buffer step can have run: it needs a reset)
+  }
+  e->obs_format = format;
+  return PGTG_OK;
+}
+
+extern "C" int pgtg_unpack_bits(pgtg_env* e, const uint32_t* bits_dev, int64_t slots, const int64_t* index_dev, int64_t count, int format,
+                                void* out_dev, const int32_t* plane_order, const int32_t* position_dev, const int32_t* velocity_dev,
+                                const int32_t* nsd_dev, void* stream) {
+  if (!e) return fail(PGTG_ERR_INVALID, "null handle");
+  if (!bk_has_obs_bits) return fail(PGTG_ERR_INVALID, "this backend has no unpack kernel");
+  if (format != PGTG_UNPACK_INT8 && format != PGTG_UNPACK_FLAT) return fail(PGTG_ERR_INVALID, "unknown unpack format (PGTG_UNPACK_INT8 or PGTG_UNPACK_FLAT)");
+  if (slots < 1 || count < 0) return fail(PGTG_ERR_INVALID, "slots must be >= 1 and count >= 0");
+  if (count && (!bits_dev || !out_dev)) return fail(PGTG_ERR_INVALID, "null argument");
+  if (format == PGTG_UNPACK_INT8 && count && ((uintptr_t)out_dev & 31)) return fail(PGTG_ERR_INVALID, "the int8 output must be 32-byte aligned");
+  int order[PGTG_MAX_CHANNELS] = {0};
+  if (format == PGTG_UNPACK_FLAT) {
+    if (!position_dev || !velocity_dev || (e->dc.use_nsd && !nsd_dev) || (e->dc.C && !plane_order))
+      return fail(PGTG_ERR_INVALID, "the flat format needs plane_order, position, velocity (and next_subgoal_direction when it is on)");
+    for (int i = 0; i < e->dc.C; i++) {
+      if (plane_order[i] < 0 || plane_order[i] >= e->dc.C) return fail(PGTG_ERR_INVALID, "bad plane order");
+      order[i] = plane_order[i];
+    }
+  }
+  bk_set_device(e->device);
+  UnpackArgs a;
+  a.bits = bits_dev; a.slot_words = pgtg_packed_obs_bytes(e) / 4; a.rows = slots * (int64_t)e->dc.N; a.count = count; a.index = index_dev;
+  a.N = e->dc.N; a.position = position_dev; a.velocity = velocity_dev; a.nsd = nsd_dev; a.err = e->unpack_err;
+  if (bk_unpack_bits(e, a, format, out_dev, order, stream)) return fail(PGTG_ERR_CUDA, std::string("unpack launch failed: ") + bk_error());
+  e->launches++;
+  return PGTG_OK;
+}
+
+extern "C" int pgtg_expand_obs(pgtg_env* e, int final, void* stream) {
+  if (!e) return fail(PGTG_ERR_INVALID, "null handle");
+  if (e->obs_format != PGTG_OBS_BITS) return fail(PGTG_ERR_STATE, "the handle stores int8 observations (pgtg_set_obs_format)");
+  if (final && !e->dc.write_final_obs) return fail(PGTG_ERR_STATE, "config was not created with write_final_obs");
+  return pgtg_unpack_bits(e, final ? e->dp.f_obs_packed : e->dp.obs_packed, 1, nullptr, e->dc.N, PGTG_UNPACK_INT8, obs_map_of(e, final != 0),
+                          nullptr, nullptr, nullptr, nullptr, stream);
 }
 
 extern "C" int64_t pgtg_launch_count(pgtg_env* e) { return e ? e->launches : 0; }

@@ -253,6 +253,7 @@ struct DevPtrs {
   const pgtg_rule* rules;
   // outputs
   uint32_t* obs_packed;  // [ceil(N * obs_bits / 32)] the observation planes as bits (env i at bit i * obs_bits), or null
+                         // (allocated by the bits observation format, or by the first host-buffer step with bits)
   int8_t* obs_map; int32_t* obs_position; int32_t* obs_velocity; int32_t* obs_nsd;
   double* reward; double* cost; uint8_t* terminated; uint8_t* truncated;
   int32_t* step_state; uint8_t* step_flags;
@@ -261,6 +262,9 @@ struct DevPtrs {
   // level sets: the pool, built once by pgtg_create (configuration, not state)
   uint16_t* level_tiles;  // [M][T] descriptors, no subgoal consumed
   uint32_t* level_plan;   // [M] plan words, start-square bits clear
+  // the bits observation format (pgtg_set_obs_format): obs_map and f_obs_map are null, the ticks store the planes only as bits,
+  // to obs_packed and (terminal observations) here, same layout
+  uint32_t* f_obs_packed;
 };
 
 // ---------------------------------------------------------------------------------------------

@@ -42,6 +42,10 @@ struct pgtg_env {
   float* flat; int flat_dim; int flat_order[PGTG_MAX_CHANNELS];
   // host-buffer steps: packed observation bits + staging for the double-buffered copies (allocated on first use)
   uint32_t* packed_dev; unsigned char* stage_dev[2]; size_t stage_bytes; void* copy_stream; void* ev_stage[2]; void* ev_copied[2]; uint64_t host_steps;
+  // observation format (pgtg_set_obs_format): in bits mode dp.obs_map / dp.f_obs_map are null and the int8 buffers live here,
+  // written by pgtg_expand_obs only; the bits buffers are state allocations
+  int obs_format; int8_t* obs_map_buf; int8_t* f_obs_map_buf; uint32_t* obs_packed_buf; uint32_t* f_obs_packed_buf;
+  uint32_t* unpack_err;  // device word: error flag 256 of pgtg_unpack_bits (pgtg_error_summary)
   int32_t* info_dev;    // [7][N] scratch of pgtg_get_info, allocated on first use
   double* stats_rows;   // [nblk][8] per-CTA episode statistics (CUDA backend)
   // device scratch for reset arguments and host-buffer steps

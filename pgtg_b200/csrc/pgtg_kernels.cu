@@ -61,6 +61,8 @@ static int bk_error_or(pgtg_env*, uint32_t* out_dev);
 #define PGTG_BACKEND_LEVELS
 static int bk_serve_levels(pgtg_env*, void* stream);
 static int bk_levels(pgtg_env*, int32_t* out_dev, int previous, void* stream);
+#define PGTG_BACKEND_OBS_BITS
+static int bk_unpack_bits(pgtg_env*, const pgtg::UnpackArgs& a, int format, void* out_dev, const int* plane_order, void* stream);
 static int bk_conn_table_max_bits() { return 24; }
 static bool bk_inline_mapgen() { return true; }
 static int bk_build_conn_table(pgtg_env*, uint32_t* table_dev);
@@ -173,6 +175,39 @@ __global__ void __launch_bounds__(256) pgtg_levels_kernel(const __grid_constant_
   for (int env = blockIdx.x * blockDim.x + threadIdx.x; env < c.N; env += gridDim.x * blockDim.x) out[env] = env_level(c, p, env, previous);
 }
 
+// pgtg_unpack_bits, int8 format: one thread per 32 output cells (unpack_chunk), expanded with the tick's byte -> 8 cells table and
+// stored as one 256-bit vector, consecutive threads -> consecutive vectors (the output is 32-byte aligned)
+__global__ void __launch_bounds__(256) pgtg_unpack_int8_kernel(const UnpackArgs a, int obs_bits, int8_t* __restrict__ out) {
+  __shared__ uint2 lut[256];
+  for (int i = threadIdx.x; i < 256; i += blockDim.x) { uint2 v; v.x = spread4((uint32_t)i); v.y = spread4((uint32_t)i >> 4); lut[i] = v; }
+  __syncthreads();
+  const uint64_t total = (uint64_t)a.count * (uint64_t)obs_bits, n32 = total / 32u, nchunks = (total + 31u) / 32u;
+  bool bad = false;
+  for (uint64_t j = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; j < nchunks; j += (uint64_t)gridDim.x * blockDim.x) {
+    const uint32_t w = unpack_chunk(a, obs_bits, j, &bad);
+    if (j < n32) pg_store_streaming32(out + 32u * j, lut[w & 255u], lut[(w >> 8) & 255u], lut[(w >> 16) & 255u], lut[w >> 24]);
+    else for (uint64_t b = 32u * j; b < total; b++) out[b] = (int8_t)((w >> (uint32_t)(b - 32u * j)) & 1u);
+  }
+  if (bad) atomicOr(a.err, PGTG_UNPACK_INDEX_ERROR);
+}
+
+// pgtg_unpack_bits, flat format: one warp per output row, the planes in sorted-key order (a lane per cell), then the scalars
+__global__ void __launch_bounds__(256) pgtg_unpack_flat_kernel(const __grid_constant__ DevCfg c, const UnpackArgs a, const __grid_constant__ FlatOrder order,
+                                                              float* __restrict__ out, int dim) {
+  const int lane = threadIdx.x & 31, PP = c.P * c.P;
+  bool bad = false;
+  for (int64_t o = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); o < a.count; o += (int64_t)gridDim.x * (blockDim.x >> 5)) {
+    const int64_t r = unpack_source_row(a, o);
+    bad |= r < 0;
+    const uint64_t bit0 = r >= 0 ? unpack_row_bit0(a, c.obs_bits, r) : 0u;
+    float* row = out + o * dim;
+    for (int k = 0; k < c.C; k++)
+      for (int cell = lane; cell < PP; cell += 32) row[k * PP + cell] = unpack_flat_cell(c, a, order.plane, r, bit0, k, cell);
+    for (int q = lane; q < dim - c.C * PP; q += 32) row[c.C * PP + q] = unpack_flat_tail(c, a, r, q);
+  }
+  if (bad && lane == 0) atomicOr(a.err, PGTG_UNPACK_INDEX_ERROR);
+}
+
 __global__ void pgtg_reduce_stats_kernel(const double* __restrict__ rows, int nrows, double* __restrict__ out) {
   // out[k] = sum over CTAs of rows[.][k]; one warp per statistic
   int k = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -256,6 +291,20 @@ static int bk_serve_levels(pgtg_env* e, void* stream) {
 static int bk_levels(pgtg_env* e, int32_t* out_dev, int previous, void* stream) {
   const int blocks = (e->dc.N + 255) / 256;
   pgtg::pgtg_levels_kernel<<<blocks < 148 * 8 ? blocks : 148 * 8, 256, 0, (cudaStream_t)stream>>>(e->dc, e->dp, previous, out_dev);
+  return ck(cudaGetLastError());
+}
+static int bk_unpack_bits(pgtg_env* e, const pgtg::UnpackArgs& a, int format, void* out_dev, const int* plane_order, void* stream) {
+  if (a.count == 0) return 0;
+  if (format == PGTG_UNPACK_INT8) {
+    const uint64_t chunks = ((uint64_t)a.count * (uint64_t)e->dc.obs_bits + 31u) / 32u, want = (chunks + 255u) / 256u;
+    if (!chunks) return 0;
+    pgtg::pgtg_unpack_int8_kernel<<<(int)(want < 148u * 16u ? want : 148u * 16u), 256, 0, (cudaStream_t)stream>>>(a, e->dc.obs_bits, (int8_t*)out_dev);
+  } else {
+    pgtg::FlatOrder order;
+    for (int i = 0; i < PGTG_MAX_CHANNELS; i++) order.plane[i] = i < e->dc.C ? plane_order[i] : 0;
+    const int64_t want = (a.count + 7) / 8;
+    pgtg::pgtg_unpack_flat_kernel<<<(int)(want < 148 * 32 ? want : 148 * 32), 256, 0, (cudaStream_t)stream>>>(e->dc, a, order, (float*)out_dev, pgtg::unpack_flat_dim(e->dc));
+  }
   return ck(cudaGetLastError());
 }
 static int bk_stats_reset(pgtg_env* e, void* stream) {

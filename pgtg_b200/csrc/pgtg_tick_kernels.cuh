@@ -114,7 +114,7 @@ __global__ void __launch_bounds__(128, LEAN ? PGTG_LEAN_MIN_BLOCKS : PGTG_MIN_BL
         if (lane == 0) sh.counters[16 + warp] = (int)any;
         if (done) phase_emit_regs<true, SLIDE>(c, p, sh, tid, env, true, er);
         __syncthreads();
-        phase_expand_final_vec(c, p.f_obs_map, sh, tid, B, env0, nvalid, sh.counters + 16);
+        phase_expand_final_vec(c, p.f_obs_map, sh, tid, B, env0, nvalid, sh.counters + 16, p.f_obs_packed);
         __syncthreads();
         {
           uint4 z; z.x = z.y = z.z = z.w = 0;
@@ -204,7 +204,7 @@ __global__ void __launch_bounds__(128, LEAN ? PGTG_LEAN_MIN_BLOCKS : PGTG_MIN_BL
   if (MODE == MODE_STEP && c.write_final_obs && n_done) {  // CTA-uniform condition
     if (done) phase_emit(c, p, sh, tid, env, true);
     __syncthreads();
-    phase_expand_final(c, p.f_obs_map, sh, tid, B, env0, n_done);
+    phase_expand_final(c, p.f_obs_map, sh, tid, B, env0, n_done, p.f_obs_packed, nvalid);
     __syncthreads();
     for (int i = tid; i < sh.bits_words; i += B) sh.bits[i] = 0;
     __syncthreads();

@@ -116,7 +116,7 @@ __global__ void __launch_bounds__(NT, MINB) pgtg_traffic_tick_kernel(const __gri
       for (int i = tid; i < nvalid * c.C * c.P; i += NT) if (sh.env[i / (c.C * c.P)].done) tk_sliding_column(c, sh, i / (c.C * c.P), i % (c.C * c.P));
     if (done) { tk_emit(c, p, sh, tid, env, true); sh.env[tid].ng_key = 0xFFFFFFFFu; }
     __syncthreads();
-    phase_expand_final(c, p.f_obs_map, bs, tid, NT, env0, n_done);
+    phase_expand_final(c, p.f_obs_map, bs, tid, NT, env0, n_done, p.f_obs_packed, nvalid);
     __syncthreads();
     for (int i = tid; i < sh.bits_words; i += NT) sh.bits[i] = 0;
     __syncthreads();

@@ -34,6 +34,8 @@ class RawEnv:
         radius = max(c.map_w, c.map_h) * 9 + 2
         lut = np.ascontiguousarray(direction_lut(radius))
         _lib.check(self.lib, self.lib.pgtg_load_direction_lut(self._h, lut.ctypes.data, radius))
+        if hc.observation_format != "int8":
+            self.set_obs_format(hc.observation_format)
         self._keep = []
 
     # -- control ------------------------------------------------------------------------------
@@ -201,6 +203,28 @@ class RawEnv:
         import torch
 
         return torch.from_dlpack(self.dlpack_capsule("level_tiles")), torch.from_dlpack(self.dlpack_capsule("level_plan"))
+
+    # -- bits observation format ---------------------------------------------------------------------------------
+    def set_obs_format(self, fmt: str):
+        """"int8" (the default) or "bits": how the ticks store the observation planes; only before the first reset."""
+        if fmt not in _lib.OBS_FORMATS:
+            raise ValueError(f"observation format must be one of {tuple(_lib.OBS_FORMATS)}")
+        _lib.check(self.lib, self.lib.pgtg_set_obs_format(self._h, _lib.OBS_FORMATS[fmt]))
+        self.hc.observation_format = fmt
+
+    def expand_obs(self, final: bool = False, stream: int = 0):
+        """Bits format: fill obs_map (final_obs_map) from obs_packed (final_obs_packed) on `stream`."""
+        _lib.check(self.lib, self.lib.pgtg_expand_obs(self._h, int(bool(final)), stream))
+
+    def unpack_bits(self, bits_ptr: int, slots: int, index_ptr: int | None, count: int, fmt: str, out_ptr: int,
+                    position_ptr: int | None = None, velocity_ptr: int | None = None, nsd_ptr: int | None = None, stream: int = 0):
+        """pgtg_unpack_bits on raw device pointers; fmt "int8" or "flat" (planes in sorted-key order, as `flatten`)."""
+        if fmt not in _lib.UNPACK_FORMATS:
+            raise ValueError(f"unpack format must be one of {tuple(_lib.UNPACK_FORMATS)}")
+        keys = self.hc.observation_keys
+        order = np.array([keys.index(k) for k in sorted(keys)] or [0], np.int32)
+        _lib.check(self.lib, self.lib.pgtg_unpack_bits(self._h, bits_ptr, int(slots), index_ptr, int(count), _lib.UNPACK_FORMATS[fmt], out_ptr,
+                                                       order.ctypes.data, position_ptr, velocity_ptr, nsd_ptr, stream))
 
     def dlpack_capsule(self, name: str):
         """-> a PyCapsule named "dltensor" for `torch.from_dlpack` / any DLPack consumer."""

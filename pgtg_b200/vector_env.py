@@ -17,7 +17,7 @@ by the native handle -- valid until the next `step`/`reset`; clone what must out
 """
 from __future__ import annotations
 
-from collections.abc import MutableMapping
+from collections.abc import Mapping, MutableMapping
 from typing import Any
 
 import numpy as np
@@ -66,6 +66,34 @@ class LazyInfo(MutableMapping):
         return f"LazyInfo({dict(self)!r})"
 
 
+class LazyPlanes(Mapping):
+    """`obs["map"]` of the bits observation format: the planes are expanded from the stored bits into the int8 buffer by one
+    kernel (`pgtg_expand_obs`) on first access, then the usual per-key views of that buffer are returned. A loop that never
+    looks at the planes pays nothing. Like the int8 views, valid until the next `step`/`reset`."""
+
+    def __init__(self, keys, expand):
+        self._keys = list(keys)
+        self._expand = expand
+        self._views = None
+
+    def _get(self):
+        if self._views is None:
+            self._views = self._expand()
+        return self._views
+
+    def __getitem__(self, key):
+        return self._get()[key]
+
+    def __iter__(self):
+        return iter(self._keys)
+
+    def __len__(self):
+        return len(self._keys)
+
+    def __repr__(self):
+        return f"LazyPlanes({self._keys!r}, expanded={self._views is not None})"
+
+
 def _device_index(device) -> int:
     d = torch.device(device)
     if d.type != "cuda":
@@ -100,6 +128,7 @@ class PGTGVectorEnv:
             self._actions = torch.zeros(num_envs, dtype=torch.int32, device=self.device)
         if conformance_draws is not None:
             self.raw.load_draws(*conformance_draws)
+        self.observation_format = self.hc.observation_format
         self._terminated = self._t["terminated"].view(torch.bool)
         self._truncated = self._t["truncated"].view(torch.bool)
 
@@ -127,10 +156,19 @@ class PGTGVectorEnv:
     def _observation(self, final: bool = False) -> dict:
         pre = "final_" if final else ""
         m = self._t[pre + "obs_map"]
+        keys = self.hc.observation_keys
+        if self.observation_format == "bits":
+            def expand():
+                with torch.cuda.device(self.device):
+                    self.raw.expand_obs(final, self._stream())
+                return {k: m[:, i] for i, k in enumerate(keys)}
+            planes = LazyPlanes(keys, expand)
+        else:
+            planes = {k: m[:, i] for i, k in enumerate(keys)}
         obs = {
             "position": self._t[pre + "obs_position"],
             "velocity": self._t[pre + "obs_velocity"],
-            "map": {k: m[:, i] for i, k in enumerate(self.hc.observation_keys)},
+            "map": planes,
         }
         if self.use_next_subgoal_direction:
             obs["next_subgoal_direction"] = self._t[pre + "obs_next_subgoal_direction"]
@@ -304,6 +342,67 @@ class PGTGVectorEnv:
                 self._t["obs_flat"] = torch.from_dlpack(self.raw.dlpack_capsule("obs_flat"))
         return self._t["obs_flat"]
 
+    # ---- bits observation format ------------------------------------------------------------------------------------
+    def obs_packed(self) -> torch.Tensor:
+        """observation_format="bits": the step's observation planes as stored by the tick, uint32 [ceil(N * C*P*P / 32)] on the
+        device, env i at bit i * C*P*P (a view, valid until the next step: copy it into a rollout store to keep it)."""
+        return self._packed_view("obs_packed")
+
+    def final_obs_packed(self) -> torch.Tensor:
+        """observation_format="bits" with final_observation=True: the terminal observations, same layout as `obs_packed`; rows
+        of envs that did not finish in the last step are not meaningful."""
+        return self._packed_view("final_obs_packed")
+
+    def _packed_view(self, name: str) -> torch.Tensor:
+        if self.observation_format != "bits":
+            raise RuntimeError(f"{name}() needs observation_format='bits'")
+        if name not in self._t:
+            with torch.cuda.device(self.device):
+                self._t[name] = torch.from_dlpack(self.raw.dlpack_capsule(name))
+        return self._t[name]
+
+    def unpack(self, bits: torch.Tensor, index: torch.Tensor | None = None, format: str = "int8", position: torch.Tensor | None = None,
+               velocity: torch.Tensor | None = None, next_subgoal_direction: torch.Tensor | None = None) -> torch.Tensor:
+        """Stored bits -> a new device tensor, one kernel, no host synchronisation. `bits`: S step slots of `obs_packed` copies
+        (a [S, words] or [words] uint32 / int32 tensor); row r = s * N + i is env i of slot s. `index`: int64 rows to gather
+        (default: all S * N in order). format="int8": [count, C, P, P] like obs["map"]; format="flat": float32 [count, D] like
+        `flat_observation()`, with `position` / `velocity` ([S, N, 2] int32) and, when next_subgoal_direction is on,
+        `next_subgoal_direction` ([S, N] int32) gathered with the same rows. A row outside [0, S * N) comes back as zeros and
+        sets an error flag that `episode_stats` reports."""
+        if format not in ("int8", "flat"):
+            raise ValueError("format must be 'int8' or 'flat'")
+        words = self.raw.packed_obs_bytes() // 4
+
+        def dev(t, dtypes, what):
+            if not (isinstance(t, torch.Tensor) and t.device == self.device and t.dtype in dtypes and t.is_contiguous()):
+                raise ValueError(f"{what} must be a contiguous {'/'.join(map(str, dtypes))} tensor on {self.device}")
+            return t
+
+        dev(bits, (torch.uint32, torch.int32), "bits")
+        if bits.numel() == 0 or bits.numel() % words:
+            raise ValueError(f"bits must hold S slots of {words} words")
+        slots, N = bits.numel() // words, self.num_envs
+        count = slots * N
+        if index is not None:
+            count = dev(index, (torch.int64,), "index").numel()
+        ptrs = [None, None, None]
+        if format == "flat":
+            needed = [(position, "position", 2), (velocity, "velocity", 2)]
+            if self.use_next_subgoal_direction:
+                needed.append((next_subgoal_direction, "next_subgoal_direction", 1))
+            for k, (t, what, per) in enumerate(needed):
+                if t is None or dev(t, (torch.int32,), what).numel() != slots * N * per:
+                    raise ValueError(f"format='flat' needs {what} as int32 [{slots}, {N}{', 2' if per == 2 else ''}]")
+                ptrs[k] = t.data_ptr()
+            C, P = self.hc.pod.num_channels, self.hc.window
+            out = torch.empty((count, C * P * P + (9 if self.use_next_subgoal_direction else 0) + 20), dtype=torch.float32, device=self.device)
+        else:
+            out = torch.empty((count, self.hc.pod.num_channels, self.hc.window, self.hc.window), dtype=torch.int8, device=self.device)
+        with torch.cuda.device(self.device):
+            self.raw.unpack_bits(bits.data_ptr(), slots, None if index is None else index.data_ptr(), count, format, out.data_ptr(),
+                                 *ptrs, stream=self._stream())
+        return out
+
     def save_map(self, path: str, env_index: int = 0) -> None:
         """EpisodeMap.save_map (map.py:173-184): the current map plan of one env as reference JSON."""
         import json
@@ -412,7 +511,8 @@ class PGTGVectorEnv:
         if flags:
             names = {1: "conformance tape overrun", 2: "conformance tape tag mismatch", 4: "conformance index out of range", 8: "goal unreachable",
                      16: "no route at a spawn square", 32: "more cars than max_cars", 64: "no start square",
-                     128: "an action outside 0..8 was replaced by the no-op 4 (the reference raises KeyError)"}
+                     128: "an action outside 0..8 was replaced by the no-op 4 (the reference raises KeyError)",
+                     256: "an unpack index outside the stored rows (its output row is zeros)"}
             raise RuntimeError("env error flags: " + "; ".join(v for k, v in names.items() if flags & k))
         v = s.cpu().tolist()
         n = max(v[0], 1.0)
