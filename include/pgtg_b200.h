@@ -308,9 +308,13 @@ int pgtg_save_state(pgtg_env* env, void* out, int64_t out_bytes);
 int pgtg_load_state(pgtg_env* env, const void* in, int64_t in_bytes);
 int pgtg_copy_state(pgtg_env* dst, pgtg_env* src);
 /* Evaluator statistics (ModularEvaluator.evaluate, evaluator.py:292-339): gamma > 0 switches on the per-env discounted
- * return (total += reward * pow(gamma, t), the powers evaluated on the host) and sets the episode cap to max_steps;
- * stats[6] = sum of the discounted returns of the finished episodes, stats[7] = how many of them were negative
- * (terminated = stats[3] + stats[4], over max_steps = stats[5]). gamma <= 0 switches it off. Synchronises. */
+ * return (total += reward * pow(gamma, t), the powers evaluated on the host), zeroes the running discounted returns and
+ * sets the episode cap to max_steps; stats[6] = sum of the discounted returns of the finished episodes, stats[7] = how
+ * many of them were negative (terminated = stats[3] + stats[4], over max_steps = stats[5]). gamma <= 0 switches it off
+ * and restores the configured cap (max_episode_steps of the configuration, or the one pgtg_copy_state took from its
+ * source). Evaluation does not change the state layout: blobs and copies stay compatible with handles that never
+ * evaluated, and they do not carry the discounted returns of episodes in flight (loading or copying zeroes them).
+ * Synchronises. */
 int pgtg_set_evaluation(pgtg_env* env, double gamma, int max_steps);
 /* Episode statistics are accumulated per CTA on the device. pgtg_reduce_stats sums them into the
  * 8-double `stats` buffer on `stream` without synchronising (so the host can NCCL-all-reduce that

@@ -74,6 +74,11 @@ static T* dev_alloc(pgtg_env* e, size_t count, bool zero = true) {
   if (zero) bk_memset(ptr, 0, bytes);
   return (T*)ptr;
 }
+static void dev_free(pgtg_env* e, void* ptr) {
+  for (size_t i = 0; i < e->allocs.size(); i++)
+    if (e->allocs[i] == ptr) { e->allocs.erase(e->allocs.begin() + i); break; }
+  bk_free(ptr);
+}
 
 // removable_edges order = graph-theory Graph.edges() after the add_edge calls of
 // generate_map_graph (map_generator.py:218-227): nodes in first-mention order, each node's
@@ -347,6 +352,7 @@ extern "C" int pgtg_create(const pgtg_config* cfg, int device, pgtg_env** out) {
   if (bk_set_device(device)) return fail(PGTG_ERR_CUDA, std::string("cannot select device: ") + bk_error());
   pgtg_env* e = new pgtg_env();
   e->cfg = *cfg; e->dc = dc; e->device = device; e->launches = 0;
+  e->max_steps_cfg = dc.max_episode_steps; e->gamma_cap = 0;
   e->have_fixed = e->have_tape = e->did_reset = false;
   e->cars_injected = false;
   e->timing = false; e->tev_used = 0;
@@ -927,7 +933,8 @@ extern "C" int pgtg_get_info(pgtg_env* e, int32_t* agent_direction, int32_t* cur
 
 // ---- full-state checkpoint / clone (PGTGEnv.light_step deep-copies the env, environment.py:1283-1299) ------------
 // Everything a tick reads or writes: SoA state, both ring slots and the map-request queues, car lists, RNG state
-// (numpy mode) / tape cursors, episode statistics, the output buffers, plus the host-side pipeline position.
+// (numpy mode) / tape cursors, episode statistics, the output buffers, plus the host-side pipeline position. Not the
+// evaluator's running discounted returns: loading or copying zeroes them (pgtg_set_evaluation).
 struct StateHeader { uint64_t magic, total_bytes, launch_index; int32_t parity, did_reset, cars_injected, lean, n_allocs, reserved; };
 static const uint64_t STATE_MAGIC = 0x5047544753544132ull;  // "PGTGSTA2"
 static size_t state_payload_bytes(const pgtg_env* e) { size_t n = 0; for (auto& s : e->state_allocs) n += (s.bytes + 15) & ~(size_t)15; return n; }
@@ -959,6 +966,7 @@ extern "C" int pgtg_load_state(pgtg_env* e, const void* in, int64_t in_bytes) {
   if (bk_sync(nullptr)) return fail(PGTG_ERR_CUDA, std::string("device error: ") + bk_error());
   const unsigned char* src = (const unsigned char*)in + sizeof h;
   for (auto& s : e->state_allocs) { bk_h2d(s.ptr, src, s.bytes, nullptr); src += (s.bytes + 15) & ~(size_t)15; }
+  if (e->dp.ep_disc) bk_memset(e->dp.ep_disc, 0, 8 * (size_t)e->dc.N);  // (not in the blob: see pgtg_set_evaluation)
   if (bk_sync(nullptr)) return fail(PGTG_ERR_CUDA, std::string("device error: ") + bk_error());
   e->launch_index = h.launch_index; e->dp.parity = h.parity; e->did_reset = h.did_reset != 0; e->cars_injected = h.cars_injected != 0; e->dc.lean = h.lean;
   return PGTG_OK;
@@ -978,33 +986,39 @@ extern "C" int pgtg_copy_state(pgtg_env* dst, pgtg_env* src) {
   if (bk_sync(nullptr)) return fail(PGTG_ERR_CUDA, std::string("device error: ") + bk_error());
   dst->launch_index = src->launch_index; dst->dp.parity = src->dp.parity; dst->did_reset = src->did_reset; dst->cars_injected = src->cars_injected;
   dst->dc.lean = src->dc.lean; dst->dc.num_rules = src->dc.num_rules; dst->dc.rules_without_traffic = src->dc.rules_without_traffic;
-  dst->dc.max_episode_steps = src->dc.max_episode_steps;
+  dst->max_steps_cfg = src->max_steps_cfg;  // (the evaluation cap, if any, stays with the handle that set it)
+  dst->dc.max_episode_steps = dst->dc.eval_on ? dst->dc.gamma_len : dst->max_steps_cfg;
+  if (dst->dp.ep_disc) { bk_memset(dst->dp.ep_disc, 0, 8 * (size_t)dst->dc.N); bk_sync(nullptr); }
   return PGTG_OK;
 }
 
 // ---- evaluator statistics (ModularEvaluator.evaluate, evaluator.py:292-339) ----------------------------------------
 // gamma > 0 switches on the per-env discounted return total += reward * pow(gamma, t) (t = tick of the episode) and the
 // two statistics built on it: stats[6] = sum of the discounted returns of finished episodes, stats[7] = how many of them
-// were negative. max_steps becomes the episode cap (the evaluator's "over max_steps" = truncations, stats[5]).
+// were negative. max_steps becomes the episode cap while evaluation is on (the evaluator's "over max_steps" =
+// truncations, stats[5]); switching it off restores the configured cap. The running discounted returns (ep_disc) are
+// not part of the checkpointed state: they only mean something inside one evaluation, every switch-on zeroes them, and
+// leaving them out keeps the state layout (blobs, pgtg_copy_state) the same whether or not a handle ever evaluated.
 extern "C" int pgtg_set_evaluation(pgtg_env* e, double gamma, int max_steps) {
   if (!e) return fail(PGTG_ERR_INVALID, "null handle");
   bk_set_device(e->device);
   if (bk_sync(nullptr)) return fail(PGTG_ERR_CUDA, std::string("device error: ") + bk_error());
-  if (!(gamma > 0)) { e->dc.eval_on = 0; return PGTG_OK; }
+  if (!(gamma > 0)) { e->dc.eval_on = 0; e->dc.max_episode_steps = e->max_steps_cfg; return PGTG_OK; }
   if (max_steps < 1) return fail(PGTG_ERR_INVALID, "max_steps must be >= 1");
   std::vector<double> tab((size_t)max_steps);
   for (int t = 0; t < max_steps; t++) tab[(size_t)t] = pow(gamma, (double)t);  // np.power(GAMMA, t) calls the same libm pow
-  double* td = dev_alloc<double>(e, (size_t)max_steps, false);
-  if (!td) return fail(PGTG_ERR_CUDA, std::string("device allocation failed: ") + bk_error());
-  bk_h2d(td, tab.data(), tab.size() * 8, nullptr);
-  if (!e->dp.ep_disc) {
-    e->dp.ep_disc = dev_alloc<double>(e, (size_t)e->dc.N);
-    if (!e->dp.ep_disc) return fail(PGTG_ERR_CUDA, std::string("device allocation failed: ") + bk_error());
-    e->state_allocs.push_back({e->dp.ep_disc, 8 * (size_t)e->dc.N});
-  } else bk_memset(e->dp.ep_disc, 0, 8 * (size_t)e->dc.N);
-  bk_sync(nullptr);
-  e->dp.gamma_pow = td;
-  e->dc.eval_on = 1; e->dc.gamma_len = max_steps; e->dc.max_episode_steps = max_steps; e->cfg.max_episode_steps = max_steps;
+  if (max_steps > e->gamma_cap) {  // the table grows; a shorter one reuses it
+    double* td = dev_alloc<double>(e, (size_t)max_steps, false);
+    if (!td) return fail(PGTG_ERR_CUDA, std::string("device allocation failed: ") + bk_error());
+    if (e->dp.gamma_pow) dev_free(e, (void*)e->dp.gamma_pow);
+    e->dp.gamma_pow = td; e->gamma_cap = max_steps;
+  }
+  bk_h2d((void*)e->dp.gamma_pow, tab.data(), tab.size() * 8, nullptr);
+  if (!e->dp.ep_disc && !(e->dp.ep_disc = dev_alloc<double>(e, (size_t)e->dc.N)))
+    return fail(PGTG_ERR_CUDA, std::string("device allocation failed: ") + bk_error());
+  bk_memset(e->dp.ep_disc, 0, 8 * (size_t)e->dc.N);
+  if (bk_sync(nullptr)) return fail(PGTG_ERR_CUDA, std::string("device error: ") + bk_error());
+  e->dc.eval_on = 1; e->dc.gamma_len = max_steps; e->dc.max_episode_steps = max_steps;
   return PGTG_OK;
 }
 

@@ -26,6 +26,8 @@ struct pgtg_env {
   struct StateAlloc { void* ptr; size_t bytes; };
   std::vector<StateAlloc> state_allocs;  // everything pgtg_save_state / pgtg_copy_state must carry (SoA state, rings, queues, outputs)
   bool have_fixed, have_tape, did_reset;
+  int max_steps_cfg;    // episode cap of the configuration (or adopted by pgtg_copy_state); dc.max_episode_steps is the cap in force
+  int gamma_cap;        // entries of dp.gamma_pow (pgtg_set_evaluation reuses the table while max_steps fits)
   bool cars_injected;   // pgtg_set_state put cars into the handle: the lean tick is off for good
   int nblk;             // CTAs per launch
   int stats_nrows;      // rows of stats_rows (one per CTA of the kernel with the most CTAs)
